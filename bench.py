@@ -2,6 +2,7 @@
 """bench.py -- SDF points/sec of the DISN hot path (BASELINE.json metric: 256^3 grid, 1/2/4/8 x B200).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 0|1|2|4] [--precision P]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic 137x137 images: encode (resize + VGG-16 + the folds)
 then the dense (res+1)^3 SDF grid per image (projection + multi-scale gather + two-stream MLP + /10).
@@ -20,6 +21,8 @@ epilogue; `--gather nccl` uses an NCCL gather instead), inside the timed region.
            caller-pinned buffers: the image crosses PCIe inside the step and the kernel's epilogue stores the SDF straight
            into the pinned host grid (no device staging, no trailing copy).  With N > 1 every rank writes its slab into one
            shared pinned host grid (POSIX shared memory registered with cudaHostRegister), each over its own PCIe link.
+`--dump-outputs DIR`: after the timed steps, what the last one returned is written as .npy files (see dump_outputs); the
+           inputs are seeded, so two builds run with the same arguments can be compared output for output.
 `--impl reference`: the CPU oracle restating the reference's TF graph (TF itself is not installable here), all host
            threads, reference loop structure (whole graph incl. VGG per chunk).  Each step is a bounded sample of the SAME
            workload: one full chunk as the reference executes it (config 0: the whole 2-chunk job).
@@ -207,6 +210,28 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------------------------------
+DUMP_FULL_BYTES = 32 << 20      # a grid up to this size is dumped whole; a larger one as a sample
+DUMP_SAMPLE = 1 << 21           # values in that sample (8 MiB, plus 16 MiB of indices)
+
+
+def dump_outputs(out_dir: str, grid: np.ndarray, mesh_counts=None):
+    """Writes the SDF grid [B, R, R, R] (float32) of the last timed step under out_dir, at most 64 MB in all:
+      sdf.npy                        the whole grid, when it is at most DUMP_FULL_BYTES;
+      sdf_sample.npy                 otherwise its values at DUMP_SAMPLE flat indices drawn with a fixed seed (sorted,
+      sdf_sample_index.npy           repeats possible), and those indices as float64;
+      mesh_counts.npy                config 4: [vertices, faces] of the mesh the step extracted (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    grid = np.ascontiguousarray(grid, dtype=np.float32)
+    if grid.nbytes <= DUMP_FULL_BYTES:
+        np.save(os.path.join(out_dir, "sdf.npy"), grid)
+    else:
+        idx = np.sort(np.random.default_rng(0).integers(0, grid.size, DUMP_SAMPLE))
+        np.save(os.path.join(out_dir, "sdf_sample.npy"), grid.reshape(-1)[idx])
+        np.save(os.path.join(out_dir, "sdf_sample_index.npy"), idx.astype(np.float64))
+    if mesh_counts is not None:
+        np.save(os.path.join(out_dir, "mesh_counts.npy"), np.asarray(mesh_counts, dtype=np.float64))
+
+
 def shared_pinned_grid(nfloats: int, rank: int, world: int, barrier):
     """One host float32 buffer visible to every rank, page-locked in every rank's CUDA context.  Returns (tensor, cleanup)."""
     import torch
@@ -302,6 +327,13 @@ def run_ours(args):
     def slab_view():        # [B, planes, R, R] contiguous view of this rank's result
         return slab if planes == max_planes else slab[:, :planes]
 
+    def result_grid():      # rank 0: the whole [B, R, R, R] grid the last step left in HBM, copied to the host
+        if world == 1:
+            return slab.cpu()
+        if peer:
+            return torch.from_numpy(eng.fetch(shared_ptr, (B, R, R, R)))
+        return torch.cat([g[:, :z_bounds[r + 1] - z_bounds[r]].cpu() for r, g in enumerate(gathered)], 1)
+
     assert B == 1 or world == 1, "config 2 (batch of 8) runs on one GPU; shard images, not slabs, to scale it out"
 
     def grid_and_gather():
@@ -374,6 +406,10 @@ def run_ours(args):
     ms_total = timed(step_device, args.steps)
     launches = eng.launch_count - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, result_grid().numpy(), (mesh["nv"], mesh["nf"]) if do_mc else None)
+        barrier()           # no rank writes the shared grid again before rank 0 has read it
     ms_step = ms_total / args.steps
     value = total_pts / (ms_step * 1e-3)
 
@@ -423,13 +459,7 @@ def run_ours(args):
     # the host grid now holds the e2e result: cross-check it against the device-resident one
     e2e_ok = None
     if rank == 0 and B == 1 and not do_mc:
-        if world == 1:
-            dev_grid = slab.cpu()
-        elif peer:
-            dev_grid = torch.from_numpy(eng.fetch(shared_ptr, (B, R, R, R)))
-        else:
-            dev_grid = torch.cat([g[:, :z_bounds[r + 1] - z_bounds[r]].cpu() for r, g in enumerate(gathered)], 1)
-        e2e_ok = bool(torch.equal(host_grid.view(B, R, R, R), dev_grid))
+        e2e_ok = bool(torch.equal(host_grid.view(B, R, R, R), result_grid()))
 
     if rank == 0:
         peaks = load_peaks()
@@ -515,7 +545,13 @@ def main():
                     help="nvidia-smi sampling period during the timed region (0 = one sample right after it)")
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="N > 1: how the z-slabs reach rank 0's HBM (peer = stores from the kernel epilogue over NVLink)")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="write the SDF grid of the last timed step under DIR as .npy (a seeded sample when it is large)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a sample of the job and keeps no grid")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -97,18 +97,16 @@ def test_get_loss_metrics():
     assert abs(m["sdf_loss_realvalue"] - np.mean([0.0, 0.1, 0.1])) < 1e-6
 
 
-def test_nn_distance_oracle_matches_reference_compiled_op():
-    """oracle/metrics_oracle.nn_distance == the reference's own CPU op compiled in place (oracle/_ref)."""
-    import pytest
+def test_nn_distance_oracle_matches_reference_compiled_op(golden):
+    """oracle/metrics_oracle.nn_distance == the reference's own CPU op compiled in place (oracle/_ref), through its outputs
+    at these inputs stored by tests/golden/make_golden_ref_calls.py."""
     from oracle import metrics_oracle as mo
+    g = golden["ref_op_outputs"]
     rng = np.random.default_rng(0)
     a = rng.standard_normal((3, 257, 3)).astype(np.float32)
     b = rng.standard_normal((3, 100, 3)).astype(np.float32)
     b[1, 5] = b[1, 9]                       # exact tie: the first minimum must win
-    try:
-        ref = mo.ref_nn_distance(a, b)
-    except FileNotFoundError:
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    ref = [g["cpu_nn_" + k] for k in ("dist1", "idx1", "dist2", "idx2")]
     got = mo.nn_distance(a, b)
     for g, r in zip(got, ref):
         np.testing.assert_array_equal(g, r)
@@ -128,23 +126,21 @@ def _approxmatch_golden():
     return g, sorted({k.rsplit("_", 1)[0] for k in g.files})
 
 
-def test_approx_match_oracle_matches_reference_compiled_op():
-    """oracle/metrics_oracle.approx_match / match_cost == the reference's own CPU ops compiled in place (oracle/_ref): equal
-    but for the float64 summation order and the last bit of expf (measured <= 4e-9 absolute on `match`; the bar is 2 ulp of float32
-    at 1.0, since numpy's exp differs in the last bit between SIMD code paths)."""
-    import pytest
+def test_approx_match_oracle_matches_reference_compiled_op(golden):
+    """oracle/metrics_oracle.approx_match / match_cost == the reference's own CPU ops compiled in place (oracle/_ref), through
+    their outputs at these inputs stored by tests/golden/make_golden_ref_calls.py: equal but for the float64 summation order and
+    the last bit of expf (measured <= 4e-9 absolute on `match`; the bar is 2 ulp of float32 at 1.0, since numpy's exp differs in
+    the last bit between SIMD code paths)."""
     from oracle import metrics_oracle as mo
+    g = golden["ref_op_outputs"]
     rng = np.random.default_rng(3)
-    for B, N, M in ((2, 64, 64), (1, 96, 32), (1, 40, 100), (1, 7, 1)):
+    for i, (B, N, M) in enumerate(((2, 64, 64), (1, 96, 32), (1, 40, 100), (1, 7, 1))):
         a = rng.uniform(-0.5, 0.5, (B, N, 3)).astype(np.float32)
         b = rng.uniform(-0.5, 0.5, (B, M, 3)).astype(np.float32)
-        try:
-            ref = mo.ref_approx_match(a, b)
-        except FileNotFoundError:
-            pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+        ref = g["cpu_am%d_match" % i]
         got = mo.approx_match(a, b)
         np.testing.assert_allclose(got, ref, rtol=2.5e-7, atol=2.5e-7)
-        np.testing.assert_allclose(mo.match_cost(a, b, ref), mo.ref_match_cost(a, b, ref), rtol=1e-7)
+        np.testing.assert_allclose(mo.match_cost(a, b, ref), g["cpu_am%d_cost" % i], rtol=1e-7)
         # what a point can give / take bounds its row / column mass (tf_approxmatch.cpp:25-27)
         assert (got.sum(axis=2) <= max(N, M) // N + 1e-5).all() and (got.sum(axis=1) <= max(N, M) // M + 1e-5).all()
 

@@ -241,9 +241,10 @@ def test_tf_checkpoint_reader_against_independently_assembled_bundle(tmp_path):
         ck.load_checkpoint(prefix, verify_data=True, model_variables_only=False)
 
 
-def test_bench_contract_helpers():
+def test_bench_contract_helpers(tmp_path):
     """bench.py: both arms print the same config.workload for every BASELINE config, the clock sampler degrades to a
-    one-shot sample / 'unavailable' without nvidia-smi, and the z-slab bookkeeping of the host path covers the grid."""
+    one-shot sample / 'unavailable' without nvidia-smi, the z-slab bookkeeping of the host path covers the grid, and
+    --dump-outputs writes a small grid whole and a large one as the same seeded float sample every time."""
     import importlib.util
     spec = importlib.util.spec_from_file_location("bench", os.path.join(os.path.dirname(os.path.dirname(__file__)), "bench.py"))
     bench = importlib.util.module_from_spec(spec)
@@ -261,3 +262,20 @@ def test_bench_contract_helpers():
     for world in (1, 2, 4, 8):
         b = sharding.z_bounds(257, world)
         assert sum(b[i + 1] - b[i] for i in range(world)) == 257
+    small = np.random.default_rng(1).standard_normal((1, 9, 9, 9)).astype(np.float32)
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    assert os.listdir(tmp_path / "small") == ["sdf.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "small" / "sdf.npy"), small)
+    large = np.arange(bench.DUMP_FULL_BYTES // 4 + 1, dtype=np.float32)
+    for d in ("large", "again"):
+        bench.dump_outputs(str(tmp_path / d), large, mesh_counts=(10, 20))
+    files = sorted(os.listdir(tmp_path / "large"))
+    assert files == ["mesh_counts.npy", "sdf_sample.npy", "sdf_sample_index.npy"]
+    assert sum(os.path.getsize(tmp_path / "large" / f) for f in files) <= 64 << 20
+    got = {f: np.load(tmp_path / "large" / f) for f in files}
+    assert all(v.dtype in (np.float32, np.float64) for v in got.values())
+    assert got["sdf_sample.npy"].shape == (bench.DUMP_SAMPLE,)
+    np.testing.assert_array_equal(got["sdf_sample.npy"], large[got["sdf_sample_index.npy"].astype(np.int64)])
+    np.testing.assert_array_equal(got["mesh_counts.npy"], [10, 20])
+    for f in files:
+        np.testing.assert_array_equal(np.load(tmp_path / "again" / f), got[f])
