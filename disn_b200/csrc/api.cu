@@ -54,9 +54,8 @@ int disn_create(const disn_config* cfg, disn_ctx** out) {
   c->num_sms = prop.multiProcessorCount;
   DISN_CUDA_OK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   c->own_stream = true;
-  DISN_CUDA_OK(cudaMalloc(&c->d_tm, sizeof(float) * 12 * 8));
-  DISN_CUDA_OK(cudaMalloc(&c->d_status, sizeof(int)));
-  DISN_CUDA_OK(cudaMemset(c->d_status, 0, sizeof(int)));
+  if (c->d_tm.reserve(sizeof(float) * 12 * 8) || c->d_status.reserve(sizeof(int))) return -1;
+  DISN_CUDA_OK(cudaMemset(c->d_status.get<int>(), 0, sizeof(int)));
   DISN_CUDA_OK(cudaMallocHost(&c->h_status, sizeof(int)));
   *c->h_status = 0;
   *out = c;
@@ -67,20 +66,9 @@ void disn_destroy(disn_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->cfg.device);
   cudaStreamSynchronize(c->stream);
-  encoder_free(c);
-  for (auto& kv : c->weights) cudaFree(kv.second.ptr);
-  for (float* p : {c->d_pts, c->d_pts_rot, c->d_out, c->d_uv, c->d_tm, c->d_axes})
-    if (p) cudaFree(p);
-  for (auto& kv : c->enc_tc_weights) cudaFree(kv.second);
-  if (c->tc_weights) cudaFree(c->tc_weights);
-  if (c->tc_weights_f8) cudaFree(c->tc_weights_f8);
-  if (c->d_status) cudaFree(c->d_status);
-  mc_free(c);
-  if (c->d_grid) cudaFree(c->d_grid);
-  if (c->d_mc_in) cudaFree(c->d_mc_in);
-  if (c->nn_scratch) cudaFree(c->nn_scratch);
-  if (c->dec_scratch) cudaFree(c->dec_scratch);
+  encoder_graph_reset(c);      // the captured graph holds the addresses of buffers `delete c` frees
   if (c->h_status) cudaFreeHost(c->h_status);
+  if (c->mc_totals_host) cudaFreeHost(c->mc_totals_host);
   if (c->own_stream && c->stream) cudaStreamDestroy(c->stream);
   delete c;
 }
@@ -90,7 +78,7 @@ static int check_status(disn_ctx* c) {
   const int st = *c->h_status;
   if (st == 0) return 0;
   *c->h_status = 0;
-  cudaMemsetAsync(c->d_status, 0, sizeof(int), c->stream);
+  cudaMemsetAsync(c->d_status.get<int>(), 0, sizeof(int), c->stream);
   if (st & DISN_STATUS_FP16_OVERFLOW) {
     set_error("DISN_PREC_F16F8: an MLP activation exceeded the fp16 range (65504); the result is invalid -- "
               "use DISN_PREC_BF16X3 (fp32 range) for these weights");
@@ -140,19 +128,17 @@ int disn_load_weight(disn_ctx* c, const char* name, const float* data, const int
   for (int i = 0; i < ndim; ++i) { DISN_REQUIRE(shape[i] > 0, "non-positive dim"); numel *= shape[i]; }
   DevTensor& t = c->weights[name];
   if (t.numel != numel) {
-    if (t.ptr) cudaFree(t.ptr);
-    t.ptr = nullptr;
-    DISN_CUDA_OK(cudaMalloc(&t.ptr, numel * sizeof(float)));
+    t.data.reset();
+    if (t.data.reserve(numel * sizeof(float))) return -1;
   }
   t.shape = shp;
   t.numel = numel;
-  DISN_CUDA_OK(cudaMemcpyAsync(t.ptr, data, numel * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(t.data.get<float>(), data, numel * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));   // caller-owned host buffer; ordered on the ctx stream
   c->weights_dirty = true;
   c->enc_B = 0;     // encoder products (taps, gbias, pmap) belong to the previous weights: force a new disn_encode
-  for (auto& kv : c->enc_tc_weights) cudaFree(kv.second);     // packed encoder weights follow the fp32 masters
-  c->enc_tc_weights.clear();
   encoder_graph_reset(c);    // the graph replays launches that read the old packed images
+  c->enc_tc_weights.clear();     // packed encoder weights follow the fp32 masters
   return 0;
 }
 
@@ -207,11 +193,14 @@ int disn_get_encoded(disn_ctx* c, int32_t what, float* out, int64_t out_elems) {
   static const int tapHW[5] = {224, 112, 56, 28, 14};
   const float* src = nullptr;
   int64_t n = 0, B = c->enc_B;
-  if (what == 0) { src = c->emb; n = B * c->cfg.num_classes; }
-  else if (what >= 1 && what <= 5) { src = c->taps[what - 1]; n = B * tapHW[what - 1] * tapHW[what - 1] * kTapC[what - 1]; }
-  else if (what == 6) { src = c->pmap; n = B * c->cfg.img_h * c->cfg.img_w * kHidden; }
-  else if (what == 7) { src = c->gbias; n = B * kHidden; }
-  else if (what == 8) { src = c->img_rs; n = B * c->cfg.vgg_in * c->cfg.vgg_in * 3; }
+  if (what == 0) { src = c->emb.get<float>(); n = B * c->cfg.num_classes; }
+  else if (what >= 1 && what <= 5) {
+    src = c->taps[what - 1].get<float>();
+    n = B * tapHW[what - 1] * tapHW[what - 1] * kTapC[what - 1];
+  }
+  else if (what == 6) { src = c->pmap.get<float>(); n = B * c->cfg.img_h * c->cfg.img_w * kHidden; }
+  else if (what == 7) { src = c->gbias.get<float>(); n = B * kHidden; }
+  else if (what == 8) { src = c->img_rs.get<float>(); n = B * c->cfg.vgg_in * c->cfg.vgg_in * 3; }
   DISN_REQUIRE(src, "unknown `what`");
   DISN_REQUIRE(out_elems == n, "output buffer has the wrong number of elements");
   DISN_CUDA_OK(cudaMemcpyAsync(out, src, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
@@ -219,7 +208,7 @@ int disn_get_encoded(disn_ctx* c, int32_t what, float* out, int64_t out_elems) {
   return 0;
 }
 
-static const float* W(disn_ctx* c, const std::string& n) { return c->weights.at(n).ptr; }
+static const float* W(disn_ctx* c, const std::string& n) { return c->weights.at(n).data.get<float>(); }
 
 static void fill_stream(disn_ctx* c, const std::string& p, StreamWeights& s) {
   s.w1 = W(c, p + "/fold1/conv1/weights"); s.b1 = W(c, p + "/fold1/conv1/biases");
@@ -232,14 +221,8 @@ static void fill_stream(disn_ctx* c, const std::string& p, StreamWeights& s) {
 
 }  // extern "C"
 int disn::ensure_point_scratch(disn_ctx* c, int64_t pts) {
-  if (pts <= c->scratch_pts) return 0;
-  for (float** p : {&c->d_pts, &c->d_pts_rot, &c->d_out, &c->d_uv}) { if (*p) cudaFree(*p); *p = nullptr; }
-  DISN_CUDA_OK(cudaMalloc(&c->d_pts, pts * 3 * sizeof(float)));
-  DISN_CUDA_OK(cudaMalloc(&c->d_pts_rot, pts * 3 * sizeof(float)));
-  DISN_CUDA_OK(cudaMalloc(&c->d_out, pts * sizeof(float)));
-  DISN_CUDA_OK(cudaMalloc(&c->d_uv, pts * 2 * sizeof(float)));
-  c->scratch_pts = pts;
-  return 0;
+  const size_t n = (size_t)pts * sizeof(float);
+  return (c->d_pts.reserve(n * 3) || c->d_pts_rot.reserve(n * 3) || c->d_out.reserve(n) || c->d_uv.reserve(n * 2)) ? -1 : 0;
 }
 
 // Device-visible alias of a caller buffer that is pinned (cudaHostAlloc / cudaHostRegister / torch pin_memory), else
@@ -253,18 +236,18 @@ static float* pinned_alias(const void* p) {
 }
 
 int disn::run_point_job(disn_ctx* c, PointJob& job) {
-  if (!job.gbias) job.gbias = c->gbias;
-  if (!job.pmap) job.pmap = c->pmap;
+  if (!job.gbias) job.gbias = c->gbias.get<float>();
+  if (!job.pmap) job.pmap = c->pmap.get<float>();
   job.img_h = c->cfg.img_h; job.img_w = c->cfg.img_w;
   job.clamp_max = c->cfg.clamp_max;
   job.tanh_out = c->cfg.tanh_out;
   fill_stream(c, "sdfprediction", job.g);
   fill_stream(c, "sdfprediction_imgfeat", job.l);
-  job.status = c->d_status;
+  job.status = c->d_status.get<int>();
   if (c->cfg.precision == DISN_PREC_FP32) return launch_point_fp32(c, job);
   if (launch_point_tc(c, job)) return -1;
   // the status word travels to the pinned mirror behind the kernel; whoever synchronises next checks it
-  DISN_CUDA_OK(cudaMemcpyAsync(c->h_status, c->d_status, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(c->h_status, c->d_status.get<int>(), sizeof(int), cudaMemcpyDeviceToHost, c->stream));
   return 0;
 }
 
@@ -289,21 +272,22 @@ int disn_eval_points(disn_ctx* c, const float* pts, const float* pts_rot, const 
   float* pred_alias = pinned_alias(out_pred);
   float* uv_alias = out_uv ? pinned_alias(out_uv) : nullptr;
   size_t nb = (size_t)B * N * 3 * sizeof(float);
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts, pts, nb, cudaMemcpyHostToDevice, c->stream));
-  job.pts = c->d_pts;
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts.get<float>(), pts, nb, cudaMemcpyHostToDevice, c->stream));
+  job.pts = c->d_pts.get<float>();
   if (pts_rot && pts_rot != pts) {
-    DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts_rot, pts_rot, nb, cudaMemcpyHostToDevice, c->stream));
-    job.pts_rot = c->d_pts_rot;
+    DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts_rot.get<float>(), pts_rot, nb, cudaMemcpyHostToDevice, c->stream));
+    job.pts_rot = c->d_pts_rot.get<float>();
   }
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm, trans_mat, (size_t)B * 12 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-  job.trans_mat = c->d_tm;
-  job.out_pred = pred_alias ? pred_alias : c->d_out;
-  job.out_uv = out_uv ? (uv_alias ? uv_alias : c->d_uv) : nullptr;
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm.get<float>(), trans_mat, (size_t)B * 12 * sizeof(float), cudaMemcpyHostToDevice,
+                               c->stream));
+  job.trans_mat = c->d_tm.get<float>();
+  job.out_pred = pred_alias ? pred_alias : c->d_out.get<float>();
+  job.out_uv = out_uv ? (uv_alias ? uv_alias : c->d_uv.get<float>()) : nullptr;
   if (run_point_job(c, job)) return -1;
   if (!pred_alias)
-    DISN_CUDA_OK(cudaMemcpyAsync(out_pred, c->d_out, (size_t)B * N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    DISN_CUDA_OK(cudaMemcpyAsync(out_pred, job.out_pred, (size_t)B * N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   if (out_uv && !uv_alias)
-    DISN_CUDA_OK(cudaMemcpyAsync(out_uv, c->d_uv, (size_t)B * N * 2 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    DISN_CUDA_OK(cudaMemcpyAsync(out_uv, job.out_uv, (size_t)B * N * 2 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
   return check_status(c);
 }
@@ -334,12 +318,10 @@ int disn_eval_grid(disn_ctx* c, const double* sdf_params, const float* trans_mat
   const int64_t N = (int64_t)(z1 - z0) * R * R;
   if (N == 0) return 0;
   // axis tables (host float64 linspace -> float32), uploaded per call: B*3*R floats
-  if (c->axes_R < R) {
-    if (c->d_axes) cudaFree(c->d_axes);
-    c->d_axes = nullptr;
-    DISN_CUDA_OK(cudaMalloc(&c->d_axes, (size_t)8 * 3 * R * sizeof(float)));
-    c->axes_R = R;
+  const size_t axes_bytes = (size_t)8 * 3 * R * sizeof(float);
+  if (c->d_axes.bytes() < axes_bytes) {
     c->axes_key.clear();
+    if (c->d_axes.reserve(axes_bytes)) return -1;
   }
   // re-upload only when the boxes / resolution change (keeps repeated calls free of host syncs)
   std::vector<double> key(sdf_params, sdf_params + (size_t)B * 6);
@@ -349,21 +331,23 @@ int disn_eval_grid(disn_ctx* c, const double* sdf_params, const float* trans_mat
     for (int b = 0; b < B; ++b)
       for (int a = 0; a < 3; ++a)
         linspace_f32(sdf_params[b * 6 + a], sdf_params[b * 6 + 3 + a], R, &axes[((size_t)b * 3 + a) * R]);
-    DISN_CUDA_OK(cudaMemcpyAsync(c->d_axes, axes.data(), axes.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    DISN_CUDA_OK(cudaMemcpyAsync(c->d_axes.get<float>(), axes.data(), axes.size() * sizeof(float), cudaMemcpyHostToDevice,
+                                 c->stream));
     DISN_CUDA_OK(cudaStreamSynchronize(c->stream));   // `axes` is a stack-owned staging buffer
     c->axes_key = key;
   }
 
   PointJob job{};
-  job.B = B; job.N = N; job.R = R; job.z0 = z0; job.axes = c->d_axes;
+  job.B = B; job.N = N; job.R = R; job.z0 = z0; job.axes = c->d_axes.get<float>();
   job.out_div = c->cfg.sdf_weight;   // correctly rounded r / 10 like the reference's float64 divide + float32 pack (create_sdf.py:285,299)
   if (flags & DISN_DEVICE_PTR) {
     job.trans_mat = trans_mat;
     job.out_pred = out_sdf;
     return run_point_job(c, job);
   }
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm, trans_mat, (size_t)B * 12 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-  job.trans_mat = c->d_tm;
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm.get<float>(), trans_mat, (size_t)B * 12 * sizeof(float), cudaMemcpyHostToDevice,
+                               c->stream));
+  job.trans_mat = c->d_tm.get<float>();
   if (float* alias = pinned_alias(out_sdf)) {     // pinned caller buffer: the kernel writes the host grid directly
     job.out_pred = alias;
     if (run_point_job(c, job)) return -1;
@@ -371,9 +355,9 @@ int disn_eval_grid(disn_ctx* c, const double* sdf_params, const float* trans_mat
     return check_status(c);
   }
   if (ensure_point_scratch(c, (int64_t)B * N)) return -1;
-  job.out_pred = c->d_out;
+  job.out_pred = c->d_out.get<float>();
   if (run_point_job(c, job)) return -1;
-  DISN_CUDA_OK(cudaMemcpyAsync(out_sdf, c->d_out, (size_t)B * N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(out_sdf, job.out_pred, (size_t)B * N * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
   return check_status(c);
 }
@@ -391,19 +375,6 @@ int disn_write_dist(const char* path, int32_t res, const double* bbox, const flo
   return 0;
 }
 
-// one persistent device scratch for the small evaluators (grows, freed in disn_destroy)
-static int small_scratch(disn_ctx* c, int64_t bytes, char** out) {
-  if (bytes > c->nn_scratch_bytes) {
-    if (c->nn_scratch) cudaFree(c->nn_scratch);
-  if (c->dec_scratch) cudaFree(c->dec_scratch);
-    c->nn_scratch = nullptr; c->nn_scratch_bytes = 0;
-    DISN_CUDA_OK(cudaMalloc(&c->nn_scratch, (size_t)bytes));
-    c->nn_scratch_bytes = bytes;
-  }
-  *out = static_cast<char*>(c->nn_scratch);
-  return 0;
-}
-
 int disn_cam_estimate(disn_ctx* c, const float* imgs, int32_t B, int32_t H, int32_t W, int32_t C, const float* K,
                       float* out_rt, float* out_trans_mat) {
   DISN_REQUIRE(c && imgs && out_trans_mat, "null argument");
@@ -411,11 +382,10 @@ int disn_cam_estimate(disn_ctx* c, const float* imgs, int32_t B, int32_t H, int3
   DISN_REQUIRE(B >= 1 && B <= c->cfg.max_batch, "batch exceeds max_batch of the context");
   if (encoder_run(c, imgs, B, H, W, C, false, /*embedding_only=*/true)) return -1;
   static const float kDefaultK[9] = {149.84375f, 0.f, 68.5f, 0.f, 149.84375f, 68.5f, 0.f, 0.f, 1.f};
-  char* base = nullptr;
-  if (small_scratch(c, 256 + (int64_t)B * 12 * 4 * 2, &base)) return -1;
-  float* dK = reinterpret_cast<float*>(base);
-  float* dRT = reinterpret_cast<float*>(base + 256);
-  float* dTM = dRT + (size_t)B * 12;
+  if (c->staging.reserve((9 + (size_t)B * 12 * 2) * 4 + 3 * 256)) return -1;
+  float* dK = c->staging.take<float>(9);
+  float* dRT = c->staging.take<float>((size_t)B * 12);
+  float* dTM = c->staging.take<float>((size_t)B * 12);
   DISN_CUDA_OK(cudaMemcpyAsync(dK, K ? K : kDefaultK, 9 * 4, cudaMemcpyHostToDevice, c->stream));
   if (launch_cam_heads(c, B, dK, dRT, dTM)) return -1;
   if (out_rt) DISN_CUDA_OK(cudaMemcpyAsync(out_rt, dRT, (size_t)B * 12 * 4, cudaMemcpyDeviceToHost, c->stream));
@@ -430,14 +400,13 @@ int disn_nn_distance(disn_ctx* c, const float* xyz1, const float* xyz2, int32_t 
   DISN_REQUIRE(B >= 1 && N >= 1 && M >= 1, "NnDistance requires non-empty point sets of shape (batch,#points,3)");
   DISN_CUDA_OK(cudaSetDevice(c->cfg.device));
   const size_t n1 = (size_t)B * N, n2 = (size_t)B * M;
-  char* base = nullptr;
-  if (small_scratch(c, (int64_t)((n1 + n2) * (3 + 1 + 1) * 4 + 1024), &base)) return -1;
-  float* d1 = reinterpret_cast<float*>(base);
-  float* d2 = d1 + n1 * 3;
-  float* o1 = d2 + n2 * 3;
-  float* o2 = o1 + n1;
-  int* i1 = reinterpret_cast<int*>(o2 + n2);
-  int* i2 = i1 + n1;
+  if (c->staging.reserve((n1 + n2) * (3 + 1 + 1) * 4 + 6 * 256)) return -1;
+  float* d1 = c->staging.take<float>(n1 * 3);
+  float* d2 = c->staging.take<float>(n2 * 3);
+  float* o1 = c->staging.take<float>(n1);
+  float* o2 = c->staging.take<float>(n2);
+  int* i1 = c->staging.take<int>(n1);
+  int* i2 = c->staging.take<int>(n2);
   DISN_CUDA_OK(cudaMemcpyAsync(d1, xyz1, n1 * 3 * 4, cudaMemcpyHostToDevice, c->stream));
   DISN_CUDA_OK(cudaMemcpyAsync(d2, xyz2, n2 * 3 * 4, cudaMemcpyHostToDevice, c->stream));
   if (nn_distance(c, d1, N, d2, M, B, o1, i1, o2, i2)) return -1;
@@ -470,15 +439,10 @@ int disn_write_obj(const char* path, const float* verts, int64_t n_verts, const 
 // staging of a host SDF grid for marching cubes (persistent, grows)
 static int mc_input(disn_ctx* c, const float* sdf, int32_t R, uint32_t flags, const float** d_sdf) {
   if (flags & DISN_DEVICE_PTR) { *d_sdf = sdf; return 0; }
-  const int64_t n = (int64_t)R * R * R;
-  if (n > c->mc_in_cap) {
-    if (c->d_mc_in) cudaFree(c->d_mc_in);
-    c->d_mc_in = nullptr; c->mc_in_cap = 0;
-    DISN_CUDA_OK(cudaMalloc(&c->d_mc_in, (size_t)n * sizeof(float)));
-    c->mc_in_cap = n;
-  }
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_mc_in, sdf, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-  *d_sdf = c->d_mc_in;
+  const size_t bytes = (size_t)R * R * R * sizeof(float);
+  if (c->d_mc_in.reserve(bytes)) return -1;
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_mc_in.get<float>(), sdf, bytes, cudaMemcpyHostToDevice, c->stream));
+  *d_sdf = c->d_mc_in.get<float>();
   return 0;
 }
 
@@ -525,17 +489,12 @@ int disn_eval_grid_resident(disn_ctx* c, const double* sdf_params, const float* 
   DISN_REQUIRE(sdf_res >= 1 && B >= 1, "sdf_res >= 1, B >= 1");
   DISN_CUDA_OK(cudaSetDevice(c->cfg.device));
   const int R = sdf_res + 1;
-  const int64_t n = (int64_t)B * R * R * R;
-  if (n > c->grid_cap) {
-    if (c->d_grid) cudaFree(c->d_grid);
-    c->d_grid = nullptr; c->grid_cap = 0;
-    DISN_CUDA_OK(cudaMalloc(&c->d_grid, (size_t)n * sizeof(float)));
-    c->grid_cap = n;
-  }
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm, trans_mat, (size_t)B * 12 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-  const int rc = disn_eval_grid(c, sdf_params, c->d_tm, B, sdf_res, 0, R, c->d_grid, DISN_DEVICE_PTR);
+  if (c->d_grid.reserve((size_t)B * R * R * R * sizeof(float))) return -1;
+  float* d_tm = c->d_tm.get<float>();
+  DISN_CUDA_OK(cudaMemcpyAsync(d_tm, trans_mat, (size_t)B * 12 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  const int rc = disn_eval_grid(c, sdf_params, d_tm, B, sdf_res, 0, R, c->d_grid.get<float>(), DISN_DEVICE_PTR);
   if (rc) return rc;
-  *out_dev = c->d_grid;
+  *out_dev = c->d_grid.get<float>();
   return 0;
 }
 

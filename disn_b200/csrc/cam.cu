@@ -75,7 +75,7 @@ int launch_cam_heads(disn_ctx* c, int B, const float* d_K, float* d_rt, float* d
   auto get = [&](const char* n, const float*& p) -> int {
     auto it = c->weights.find(std::string("cameraprediction/") + n);
     DISN_REQUIRE(it != c->weights.end(), std::string("missing variable cameraprediction/") + n);
-    p = it->second.ptr;
+    p = it->second.data.get<float>();
     return 0;
   };
   if (get("scale/fc1/weights", w.s1w) || get("scale/fc1/biases", w.s1b) || get("scale/fc2/weights", w.s2w) ||
@@ -87,7 +87,7 @@ int launch_cam_heads(disn_ctx* c, int B, const float* d_K, float* d_rt, float* d
       get("translation/fc3/weights", w.t3w) || get("translation/fc3/biases", w.t3b))
     return -2;
   DISN_REQUIRE(c->cfg.num_classes <= 1024, "camera heads expect an embedding of at most 1024");
-  cam_heads_kernel<<<B, 256, 0, c->stream>>>(c->emb, c->cfg.num_classes, w, d_K, d_rt, d_tm);
+  cam_heads_kernel<<<B, 256, 0, c->stream>>>(c->emb.get<float>(), c->cfg.num_classes, w, d_K, d_rt, d_tm);
   c->launches++;
   DISN_CUDA_OK(cudaGetLastError());
   return 0;

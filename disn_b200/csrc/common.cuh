@@ -6,6 +6,7 @@
 #include <map>
 #include <set>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/disn_b200.h"
@@ -32,8 +33,54 @@ void set_error(const std::string& msg);
     }                                                    \
   } while (0)
 
+// Sole owner of one cudaMalloc block (move-only; freed by the destructor).  take<T>() carves consecutive 256-byte-aligned
+// arrays off the block, starting at its base after every reserve(); each array wastes under 256 bytes of padding, so a
+// block carved into k arrays needs their total size plus k * 256 bytes.
+class DevBuf {
+ public:
+  DevBuf() = default;
+  DevBuf(DevBuf&& o) noexcept { *this = std::move(o); }
+  DevBuf& operator=(DevBuf&& o) noexcept {
+    std::swap(p_, o.p_); std::swap(bytes_, o.bytes_); std::swap(used_, o.used_);
+    return *this;
+  }
+  ~DevBuf() { reset(); }
+
+  // Grow-only: a block of at least `bytes` keeps its contents, a smaller one is replaced by exactly `bytes` (contents
+  // lost).  On failure the buffer is left empty, the error recorded, and -1 returned.
+  int reserve(size_t bytes) {
+    used_ = 0;
+    if (bytes <= bytes_) return 0;
+    reset();
+    const cudaError_t e = cudaMalloc(&p_, bytes);
+    if (e != cudaSuccess) {
+      p_ = nullptr;
+      set_error("cudaMalloc of " + std::to_string(bytes) + " bytes failed: " + cudaGetErrorString(e));
+      return -1;
+    }
+    bytes_ = bytes;
+    return 0;
+  }
+  void reset() {
+    if (p_) cudaFree(p_);
+    p_ = nullptr;
+    bytes_ = used_ = 0;
+  }
+  size_t bytes() const { return bytes_; }
+  template <class T> T* get() const { return static_cast<T*>(p_); }
+  template <class T> T* take(size_t count) {
+    T* r = reinterpret_cast<T*>(static_cast<char*>(p_) + used_);
+    used_ += (count * sizeof(T) + 255) / 256 * 256;
+    return r;
+  }
+
+ private:
+  void* p_ = nullptr;
+  size_t bytes_ = 0, used_ = 0;
+};
+
 struct DevTensor {
-  float* ptr = nullptr;
+  DevBuf data;
   std::vector<int64_t> shape;
   int64_t numel = 0;
 };
@@ -103,50 +150,44 @@ struct disn_ctx {
 
   // encoder state
   int32_t enc_B = 0;
-  int32_t alloc_B = 0;
-  float* img_in = nullptr;      // [B,H,W,3] as uploaded
-  float* img_rs = nullptr;      // [B,224,224,3]
-  float* act[2] = {nullptr, nullptr};   // ping-pong activations
-  float* taps[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-  float* proj[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // per-level projected maps [B,h,h,512]
-  float* fc_a = nullptr;        // [B,4096]
-  float* fc_b = nullptr;        // [B,4096]
-  float* partial = nullptr;     // split-K partials (fc layers)
-  float* splitk_ws = nullptr;   // split-K partials (conv / projection GEMMs)
-  int64_t splitk_ws_elems = 0;
-  float* emb = nullptr;         // [B,num_classes]
-  float* gbias = nullptr;       // [B,512]
-  float* pmap = nullptr;        // [B,img_h,img_w,512]
+  int32_t alloc_B = 0;          // batch the encoder buffers below are sized for
+  disn::DevBuf img_in;          // [B,H,W,3] as uploaded
+  disn::DevBuf img_rs;          // [B,224,224,3]
+  disn::DevBuf act[2];          // ping-pong activations
+  disn::DevBuf taps[5];
+  disn::DevBuf proj[5];         // per-level projected maps [B,h,h,512]
+  disn::DevBuf fc_a, fc_b;      // [B,4096]
+  disn::DevBuf partial;         // split-K partials (fc layers)
+  disn::DevBuf splitk_ws;       // split-K partials (conv / projection GEMMs)
+  disn::DevBuf emb;             // [B,num_classes]
+  disn::DevBuf gbias;           // [B,512]
+  disn::DevBuf pmap;            // [B,img_h,img_w,512]
   cudaGraphExec_t enc_graph_exec = nullptr;   // captured encoder launch sequence (encoder_run)
   std::vector<int64_t> enc_graph_key, enc_warm_key;
   int64_t enc_graph_launches = 0;
-  // scratch for host-pointer calls
-  float* d_pts = nullptr; float* d_pts_rot = nullptr; float* d_out = nullptr; float* d_uv = nullptr;
-  int64_t scratch_pts = 0;
-  float* d_tm = nullptr;        // [max_batch,4,3]
-  int* d_status = nullptr;      // device status word (PointJob::status)
+  // scratch for host-pointer calls (ensure_point_scratch)
+  disn::DevBuf d_pts, d_pts_rot, d_out, d_uv;
+  disn::DevBuf d_tm;            // [max_batch,4,3]
+  disn::DevBuf d_status;        // device status word (PointJob::status)
   int* h_status = nullptr;      // pinned host mirror, copied behind every point-kernel launch
-  float* d_axes = nullptr;      // [max_batch,3,R]
-  int32_t axes_R = 0;
+  disn::DevBuf d_axes;          // [max_batch,3,R]
   std::vector<double> axes_key; // (sdf_params, R) the tables in d_axes were built from
   // bf16x3 packed weights (tcgen05 path)
-  void* tc_weights = nullptr;          // bf16 hi/lo stage images of the point MLP (DISN_PREC_BF16X3)
-  int64_t tc_weights_bytes = 0;
-  void* tc_weights_f8 = nullptr;       // fp16 + e5m2 stage images (DISN_PREC_F16F8)
+  disn::DevBuf tc_weights;             // bf16 hi/lo stage images of the point MLP (DISN_PREC_BF16X3)
+  disn::DevBuf tc_weights_f8;          // fp16 + e5m2 stage images (DISN_PREC_F16F8)
   float tc_act_scale[2][4][2] = {};
   float tc_small[2][2048] = {};         // host copy of the per-stream small parameters (the point kernel's __grid_constant__ table)
-  std::map<std::string, uint8_t*> enc_tc_weights;   // packed bf16 hi/lo stage images of the encoder GEMMs
+  std::map<std::string, disn::DevBuf> enc_tc_weights;   // packed bf16 hi/lo stage images of the encoder GEMMs
   // marching cubes: persistent scratch + the device-resident mesh of the last run (mc.cu)
-  uint8_t* mc_code = nullptr; uint32_t* mc_vbase = nullptr; uint32_t* mc_chunk = nullptr; uint32_t* mc_sums = nullptr;
-  uint32_t* mc_totals = nullptr; uint32_t* mc_totals_host = nullptr;
-  float* mc_verts = nullptr; int32_t* mc_faces = nullptr;
-  int64_t mc_pts_cap = 0, mc_verts_cap = 0, mc_faces_cap = 0, mc_nv = 0, mc_nf = 0;
+  disn::DevBuf mc_code, mc_vbase, mc_chunk, mc_sums, mc_totals;
+  uint32_t* mc_totals_host = nullptr;   // pinned
+  disn::DevBuf mc_verts, mc_faces;
+  int64_t mc_nv = 0, mc_nf = 0;
   // device-resident SDF grid of disn_eval_grid_resident and host staging for the marching-cubes input
-  float* d_grid = nullptr; int64_t grid_cap = 0;
-  float* d_mc_in = nullptr; int64_t mc_in_cap = 0;
-  // nn_distance / cam scratch (persistent, grows)
-  void* nn_scratch = nullptr; int64_t nn_scratch_bytes = 0;
-  void* dec_scratch = nullptr; int64_t dec_scratch_bytes = 0;   // explicit-feature decoder staging (decoder.cu)
+  disn::DevBuf d_grid;
+  disn::DevBuf d_mc_in;
+  // staging of the host-pointer calls that synchronise before they return (nn_distance, cam, explicit-feature decoder)
+  disn::DevBuf staging;
 };
 
 namespace disn {
@@ -154,7 +195,6 @@ namespace disn {
 int encoder_alloc(disn_ctx* c, int B);
 int encoder_run(disn_ctx* c, const float* imgs, int B, int H, int W, int C, bool device_ptr,
                 bool embedding_only = false);
-void encoder_free(disn_ctx* c);
 void encoder_graph_reset(disn_ctx* c);
 // api.cu
 int run_point_job(disn_ctx* c, PointJob& job);    // fills weights / encoder products / status and launches per cfg.precision
@@ -169,7 +209,7 @@ int launch_point_fp32(disn_ctx* c, const PointJob& job);
 int tc_pack_weights(disn_ctx* c);
 int launch_point_tc(disn_ctx* c, const PointJob& job);
 // conv_tc.cu
-int conv_tc_pack(disn_ctx* c, const float* d_w, int K, int N, uint8_t** out_dev);
+int conv_tc_pack(disn_ctx* c, const float* d_w, int K, int N, DevBuf& out);
 int launch_conv_tc(disn_ctx* c, const float* A, const uint8_t* wpk, const float* bias, float* C, float* ws,
                    int64_t ws_elems, int M, int N, int K, int H, int W, int Cin, int relu, int* splits_out);
 // cam.cu
@@ -180,5 +220,4 @@ int nn_distance(disn_ctx* c, const float* d_xyz1, int n, const float* d_xyz2, in
 // mc.cu
 int mc_run(disn_ctx* c, const float* d_sdf, int R, const double* bbox, float iso, int64_t* n_verts, int64_t* n_faces);
 int mc_fetch(disn_ctx* c, float* verts, int32_t* faces);
-void mc_free(disn_ctx* c);
 }  // namespace disn

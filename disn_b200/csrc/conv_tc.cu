@@ -317,7 +317,7 @@ __global__ void __launch_bounds__(CT_THREADS, 1) conv_tc_kernel(ConvTcJob job, u
 }  // namespace
 
 // [K, N] fp32 row-major (device) -> packed B stage images [N/128][K/64][hi|lo][128 x 64 SW128 bf16] (device)
-int conv_tc_pack(disn_ctx* c, const float* d_w, int K, int N, uint8_t** out_dev) {
+int conv_tc_pack(disn_ctx* c, const float* d_w, int K, int N, DevBuf& out) {
   std::vector<float> w((size_t)K * N);
   DISN_CUDA_OK(cudaMemcpyAsync(w.data(), d_w, w.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
@@ -337,8 +337,8 @@ int conv_tc_pack(disn_ctx* c, const float* d_w, int K, int N, uint8_t** out_dev)
       }
   // copy on the context's (non-blocking) stream and wait: a plain cudaMemcpy from pageable memory may return before
   // the DMA has landed and is not ordered against kernels on a non-blocking stream
-  DISN_CUDA_OK(cudaMalloc(out_dev, img.size()));
-  DISN_CUDA_OK(cudaMemcpyAsync(*out_dev, img.data(), img.size(), cudaMemcpyHostToDevice, c->stream));
+  if (out.reserve(img.size())) return -1;
+  DISN_CUDA_OK(cudaMemcpyAsync(out.get<void>(), img.data(), img.size(), cudaMemcpyHostToDevice, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
   return 0;
 }
@@ -376,15 +376,14 @@ int launch_conv_tc(disn_ctx* c, const float* A, const uint8_t* wpk, const float*
   if (!measure) {
     conv_tc_kernel<false><<<grid, CT_THREADS, smem, c->stream>>>(job, nullptr);
   } else {      // diagnostics: synchronous, prints the per-role blocked time of this launch
-    unsigned long long* dbg = nullptr;
     const size_t n = (size_t)grid * 16 * (CW_NCLS + 1);
-    DISN_CUDA_OK(cudaMalloc(&dbg, n * sizeof(unsigned long long)));
-    DISN_CUDA_OK(cudaMemsetAsync(dbg, 0, n * sizeof(unsigned long long), c->stream));
-    conv_tc_kernel<true><<<grid, CT_THREADS, smem, c->stream>>>(job, dbg);
+    DevBuf dbg;
+    if (dbg.reserve(n * sizeof(unsigned long long))) return -1;
+    DISN_CUDA_OK(cudaMemsetAsync(dbg.get<void>(), 0, n * sizeof(unsigned long long), c->stream));
+    conv_tc_kernel<true><<<grid, CT_THREADS, smem, c->stream>>>(job, dbg.get<unsigned long long>());
     std::vector<unsigned long long> h(n);
     DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
-    DISN_CUDA_OK(cudaMemcpy(h.data(), dbg, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    cudaFree(dbg);
+    DISN_CUDA_OK(cudaMemcpy(h.data(), dbg.get<void>(), n * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     static const char* cls[CW_NCLS] = {"bempty", "accfree", "afull", "bfull", "accfull", "aempty"};
     static const int show[5] = {0, 1, 4, 8, 12};
     static const char* role[5] = {"Bprod", "MMA", "epi.q0", "Aprod.g0", "Aprod.g1"};

@@ -79,19 +79,6 @@ __global__ void img_points_kernel(const float* __restrict__ pts, const float* __
   }
 }
 
-int dec_scratch(disn_ctx* c, int64_t bytes, char** out) {
-  if (bytes > c->dec_scratch_bytes) {
-    if (c->dec_scratch) cudaFree(c->dec_scratch);
-    c->dec_scratch = nullptr; c->dec_scratch_bytes = 0;
-    DISN_CUDA_OK(cudaMalloc(&c->dec_scratch, (size_t)bytes));
-    c->dec_scratch_bytes = bytes;
-  }
-  *out = static_cast<char*>(c->dec_scratch);
-  return 0;
-}
-
-int64_t align256(int64_t v) { return (v + 255) / 256 * 256; }
-
 }  // namespace
 }  // namespace disn
 
@@ -110,18 +97,19 @@ int disn_point_img_feat(disn_ctx* c, const float* pts, const float* trans_mat, i
   if (N <= 0) return 0;
   static const int tapHW[5] = {224, 112, 56, 28, 14};
   const int64_t n = (int64_t)B * N;
-  char* base = nullptr;
-  if (dec_scratch(c, align256(n * 3 * 4) + align256(n * 2 * 4) + align256(n * kLocalFeat * 4) + 256, &base)) return -1;
-  float* d_pts = reinterpret_cast<float*>(base);
-  float* d_uv = reinterpret_cast<float*>(base + align256(n * 3 * 4));
-  float* d_feat = reinterpret_cast<float*>(base + align256(n * 3 * 4) + align256(n * 2 * 4));
+  if (c->staging.reserve((size_t)n * (3 + 2 + kLocalFeat) * 4 + 3 * 256)) return -1;
+  float* d_pts = c->staging.take<float>(n * 3);
+  float* d_uv = c->staging.take<float>(n * 2);
+  float* d_feat = c->staging.take<float>(n * kLocalFeat);
   DISN_CUDA_OK(cudaMemcpyAsync(d_pts, pts, (size_t)n * 3 * 4, cudaMemcpyHostToDevice, c->stream));
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm, trans_mat, (size_t)B * 12 * 4, cudaMemcpyHostToDevice, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm.get<float>(), trans_mat, (size_t)B * 12 * 4, cudaMemcpyHostToDevice, c->stream));
   const int blocks = (int)std::min<int64_t>((n + 255) / 256, (int64_t)c->num_sms * 8);
-  img_points_kernel<<<blocks, 256, 0, c->stream>>>(d_pts, c->d_tm, d_uv, B, N, c->cfg.clamp_max);
+  img_points_kernel<<<blocks, 256, 0, c->stream>>>(d_pts, c->d_tm.get<float>(), d_uv, B, N, c->cfg.clamp_max);
   TapLevels lv;
   int off = 0;
-  for (int l = 0; l < 5; ++l) { lv.p[l] = c->taps[l]; lv.h[l] = tapHW[l]; lv.c[l] = kTapC[l]; lv.coff[l] = off; off += kTapC[l]; }
+  for (int l = 0; l < 5; ++l) {
+    lv.p[l] = c->taps[l].get<float>(); lv.h[l] = tapHW[l]; lv.c[l] = kTapC[l]; lv.coff[l] = off; off += kTapC[l];
+  }
   const int64_t total = n * (kLocalFeat / 4);
   const int blocks2 = (int)std::min<int64_t>((total + 255) / 256, (int64_t)c->num_sms * 16);
   point_img_feat_kernel<<<blocks2, 256, 0, c->stream>>>(lv, d_uv, d_feat, B, N, c->cfg.img_h, c->cfg.img_w, kLocalFeat / 4);
@@ -144,27 +132,26 @@ int disn_eval_points_ex(disn_ctx* c, const float* pts, const float* pts_rot, con
   if (N <= 0) return 0;
   const int64_t n = (int64_t)B * N;
   if (ensure_point_scratch(c, n)) return -1;
-  char* base = nullptr;
-  if (dec_scratch(c, 2 * align256(n * 4) + 256, &base)) return -1;
-  float* d_g = reinterpret_cast<float*>(base);
-  float* d_l = reinterpret_cast<float*>(base + align256(n * 4));
+  if (c->staging.reserve((size_t)n * 2 * 4 + 2 * 256)) return -1;
+  float* d_g = c->staging.take<float>(n);
+  float* d_l = c->staging.take<float>(n);
   PointJob job{};
   job.B = B; job.N = N; job.out_div = 1.0f;
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts, pts, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
-  job.pts = c->d_pts;
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts.get<float>(), pts, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
+  job.pts = c->d_pts.get<float>();
   if (pts_rot && pts_rot != pts) {
-    DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts_rot, pts_rot, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
-    job.pts_rot = c->d_pts_rot;
+    DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts_rot.get<float>(), pts_rot, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
+    job.pts_rot = c->d_pts_rot.get<float>();
   }
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm, trans_mat, (size_t)B * 48, cudaMemcpyHostToDevice, c->stream));
-  job.trans_mat = c->d_tm;
-  job.out_pred = c->d_out;
-  job.out_uv = out_uv ? c->d_uv : nullptr;
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm.get<float>(), trans_mat, (size_t)B * 48, cudaMemcpyHostToDevice, c->stream));
+  job.trans_mat = c->d_tm.get<float>();
+  job.out_pred = c->d_out.get<float>();
+  job.out_uv = out_uv ? c->d_uv.get<float>() : nullptr;
   job.out_global = out_global ? d_g : nullptr;
   job.out_local = out_local ? d_l : nullptr;
   if (run_point_job(c, job)) return -1;
-  DISN_CUDA_OK(cudaMemcpyAsync(out_pred, c->d_out, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-  if (out_uv) DISN_CUDA_OK(cudaMemcpyAsync(out_uv, c->d_uv, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(out_pred, c->d_out.get<float>(), (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  if (out_uv) DISN_CUDA_OK(cudaMemcpyAsync(out_uv, c->d_uv.get<float>(), (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
   if (out_global) DISN_CUDA_OK(cudaMemcpyAsync(out_global, d_g, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
   if (out_local) DISN_CUDA_OK(cudaMemcpyAsync(out_local, d_l, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
@@ -186,41 +173,37 @@ int disn_eval_features(disn_ctx* c, const float* pts_rot, const float* global_fe
   const int nc = c->cfg.num_classes;
   const int64_t n = (int64_t)B * N;
   if (ensure_point_scratch(c, n)) return -1;
-  char* base = nullptr;
-  const int64_t o_feat = 0, o_pf = o_feat + align256(n * kLocalFeat * 4), o_gf = o_pf + align256(n * kHidden * 4),
-                o_gb = o_gf + align256((int64_t)B * nc * 4), o_g = o_gb + align256((int64_t)B * kHidden * 4),
-                o_l = o_g + align256(n * 4), o_end = o_l + align256(n * 4);
-  if (dec_scratch(c, o_end + 256, &base)) return -1;
-  float* d_feat = reinterpret_cast<float*>(base + o_feat);
-  float* d_pf = reinterpret_cast<float*>(base + o_pf);
-  float* d_gf = reinterpret_cast<float*>(base + o_gf);
-  float* d_gb = reinterpret_cast<float*>(base + o_gb);
-  float* d_g = reinterpret_cast<float*>(base + o_g);
-  float* d_l = reinterpret_cast<float*>(base + o_l);
+  if (c->staging.reserve(((size_t)n * (kLocalFeat + kHidden + 2) + (size_t)B * (nc + kHidden)) * 4 + 6 * 256)) return -1;
+  float* d_feat = c->staging.take<float>(n * kLocalFeat);
+  float* d_pf = c->staging.take<float>(n * kHidden);
+  float* d_gf = c->staging.take<float>((size_t)B * nc);
+  float* d_gb = c->staging.take<float>((size_t)B * kHidden);
+  float* d_g = c->staging.take<float>(n);
+  float* d_l = c->staging.take<float>(n);
   DISN_CUDA_OK(cudaMemcpyAsync(d_feat, point_feat, (size_t)n * kLocalFeat * 4, cudaMemcpyHostToDevice, c->stream));
   DISN_CUDA_OK(cudaMemcpyAsync(d_gf, global_feat, (size_t)B * nc * 4, cudaMemcpyHostToDevice, c->stream));
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts, pts_rot, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
-  const auto& wg = c->weights.at("sdfprediction/fold2/conv1/weights");
-  const auto& bg = c->weights.at("sdfprediction/fold2/conv1/biases");
-  const auto& wl = c->weights.at("sdfprediction_imgfeat/fold2/conv1/weights");
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_pts.get<float>(), pts_rot, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
+  const float* wg = c->weights.at("sdfprediction/fold2/conv1/weights").data.get<float>();
+  const float* bg = c->weights.at("sdfprediction/fold2/conv1/biases").data.get<float>();
+  const float* wl = c->weights.at("sdfprediction_imgfeat/fold2/conv1/weights").data.get<float>();
   // global stream: gbias = g . Wg[512:512+nc] + b      (models/sdfnet.py:78-85)
-  if (encoder_gemv(c, d_gf, wg.ptr + (int64_t)kHidden * kHidden, bg.ptr, d_gb, B, nc, kHidden, 0)) return -1;
+  if (encoder_gemv(c, d_gf, wg + (int64_t)kHidden * kHidden, bg, d_gb, B, nc, kHidden, 0)) return -1;
   // local stream: pfeat = feat . Wl[512:1984]          (models/sdfnet.py:180-183; bias added in the point kernel)
-  if (encoder_gemm_plain(c, "decoder_proj", d_feat, wl.ptr + (int64_t)kHidden * kHidden, nullptr, d_pf, (int)n, kHidden,
+  if (encoder_gemm_plain(c, "decoder_proj", d_feat, wl + (int64_t)kHidden * kHidden, nullptr, d_pf, (int)n, kHidden,
                          kLocalFeat, 0))
     return -1;
   static const float kIdentityish[12] = {1, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 1};   // q2 = 1: the unused projection stays finite
   float tm[8 * 12];
   for (int b = 0; b < B; ++b) memcpy(tm + b * 12, kIdentityish, sizeof(kIdentityish));
-  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm, tm, (size_t)B * 48, cudaMemcpyHostToDevice, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(c->d_tm.get<float>(), tm, (size_t)B * 48, cudaMemcpyHostToDevice, c->stream));
   PointJob job{};
   job.B = B; job.N = N; job.out_div = 1.0f;
-  job.pts = c->d_pts;
-  job.trans_mat = c->d_tm;
+  job.pts = c->d_pts.get<float>();
+  job.trans_mat = c->d_tm.get<float>();
   job.gbias = d_gb;
   job.pmap = d_pf;            // never dereferenced in pfeat mode
   job.pfeat = d_pf;
-  job.out_pred = c->d_out;
+  job.out_pred = c->d_out.get<float>();
   job.out_global = out_global ? d_g : nullptr;
   job.out_local = out_local ? d_l : nullptr;
   const int saved_tanh = c->cfg.tanh_out;
@@ -228,7 +211,7 @@ int disn_eval_features(disn_ctx* c, const float* pts_rot, const float* global_fe
   const int rc = run_point_job(c, job);
   c->cfg.tanh_out = saved_tanh;
   if (rc) return -1;
-  DISN_CUDA_OK(cudaMemcpyAsync(out_pred, c->d_out, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(out_pred, c->d_out.get<float>(), (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
   if (out_global) DISN_CUDA_OK(cudaMemcpyAsync(out_global, d_g, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
   if (out_local) DISN_CUDA_OK(cudaMemcpyAsync(out_local, d_l, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
   return disn_synchronize(c);

@@ -147,17 +147,6 @@ __global__ void __launch_bounds__(EM_THREADS) match_cost_sum_kernel(const double
   if (threadIdx.x == 0) cost[b] = __double2float_rn(part[0]);
 }
 
-struct DevBuf {       // one allocation, released on every exit path
-  char* base = nullptr;
-  char* p = nullptr;
-  ~DevBuf() { if (base) cudaFree(base); }
-  template <class T> T* take(size_t count) {
-    T* r = reinterpret_cast<T*>(p);
-    p += (count * sizeof(T) + 255) / 256 * 256;
-    return r;
-  }
-};
-
 int match_cost_device(disn_ctx* c, const float* d1, const float* d2, const float* dmatch, int B, int N, int M, double* rowcost,
                       float* dcost) {
   match_cost_rows_kernel<<<dim3((N + EM_WARPS - 1) / EM_WARPS, B), EM_THREADS, 0, c->stream>>>(d1, d2, dmatch, N, M, rowcost);
@@ -178,10 +167,8 @@ extern "C" int disn_approx_match(disn_ctx* c, const float* xyz1, const float* xy
   DISN_REQUIRE(B >= 1 && N >= 1 && M >= 1 && B <= 65535, "ApproxMatch expects (batch_size,num_points,3) point sets, batch <= 65535");
   DISN_CUDA_OK(cudaSetDevice(c->cfg.device));
   const size_t n1 = (size_t)B * N, n2 = (size_t)B * M, nm = (size_t)B * N * M;
-  DevBuf buf;
-  const size_t bytes = (n1 + n2) * 12 + (3 * n1 + 3 * n2) * 8 + nm * 4 + n1 * 8 + (size_t)B * 4 + 16 * 256;
-  DISN_CUDA_OK(cudaMalloc(&buf.base, bytes));
-  buf.p = buf.base;
+  DevBuf buf;       // per call: the match matrix alone is B*N*M floats
+  if (buf.reserve((n1 + n2) * 12 + (3 * n1 + 3 * n2) * 8 + nm * 4 + n1 * 8 + (size_t)B * 4 + 16 * 256)) return -1;
   float* d1 = buf.take<float>(n1 * 3);
   float* d2 = buf.take<float>(n2 * 3);
   double* satl[2] = {buf.take<double>(n1), buf.take<double>(n1)};
@@ -229,8 +216,7 @@ extern "C" int disn_match_cost(disn_ctx* c, const float* xyz1, const float* xyz2
   DISN_CUDA_OK(cudaSetDevice(c->cfg.device));
   const size_t n1 = (size_t)B * N, n2 = (size_t)B * M, nm = (size_t)B * N * M;
   DevBuf buf;
-  DISN_CUDA_OK(cudaMalloc(&buf.base, (n1 + n2) * 12 + nm * 4 + n1 * 8 + (size_t)B * 4 + 8 * 256));
-  buf.p = buf.base;
+  if (buf.reserve((n1 + n2) * 12 + nm * 4 + n1 * 8 + (size_t)B * 4 + 8 * 256)) return -1;
   float* d1 = buf.take<float>(n1 * 3);
   float* d2 = buf.take<float>(n2 * 3);
   float* dmatch = buf.take<float>(nm);

@@ -231,11 +231,11 @@ static int launch_gemm(disn_ctx* c, int mode, const float* A, const float* Bm, c
     if (want > kchunks) want = kchunks;
     for (int d = want; d >= 1; --d)
       if ((K / 8) % d == 0) { splits = d; break; }
-    if ((int64_t)splits * M * N > c->splitk_ws_elems) splits = 1;
+    if ((size_t)splits * M * N * sizeof(float) > c->splitk_ws.bytes()) splits = 1;
   }
   const int kper = (splits == 1) ? K : K / splits;
   dim3 grid(N / BN, (M + 127) / 128, splits);
-  float* ws = splits > 1 ? c->splitk_ws : nullptr;
+  float* ws = splits > 1 ? c->splitk_ws.get<float>() : nullptr;
   if (BN == 128) gemm_dispatch<128>(mode, vec, grid, c->stream, A, Bm, bias, C, M, N, K, relu, g, kper, ws);
   else gemm_dispatch<64>(mode, vec, grid, c->stream, A, Bm, bias, C, M, N, K, relu, g, kper, ws);
   c->launches++;
@@ -257,16 +257,17 @@ static int gemm_any(disn_ctx* c, const std::string& wname, int mode, const float
   const bool tc_ok = c->cfg.precision != DISN_PREC_FP32 && K % 64 == 0 && N % 32 == 0 &&
                      (mode == A_PLAIN || g.Cin % 64 == 0);
   if (!tc_ok) return launch_gemm(c, mode, A, Bm, bias, C, M, N, K, relu, g);
-  uint8_t*& pk = c->enc_tc_weights[wname];
-  if (!pk && conv_tc_pack(c, Bm, K, N, &pk)) return -1;
+  DevBuf& pk = c->enc_tc_weights[wname];
+  if (!pk.bytes() && conv_tc_pack(c, Bm, K, N, pk)) return -1;
   int splits = 1;
-  if (launch_conv_tc(c, A, pk, bias, C, c->splitk_ws, c->splitk_ws_elems, M, N, K, mode == A_IM2COL ? g.H : 0,
-                     g.W, g.Cin, relu, &splits))
+  float* ws = c->splitk_ws.get<float>();
+  if (launch_conv_tc(c, A, pk.get<uint8_t>(), bias, C, ws, c->splitk_ws.bytes() / sizeof(float), M, N, K,
+                     mode == A_IM2COL ? g.H : 0, g.W, g.Cin, relu, &splits))
     return -1;
   if (splits > 1) {
     const int64_t mn4 = (int64_t)M * N / 4;
     int blocks = (int)std::min<int64_t>((mn4 + 255) / 256, 148 * 8);
-    splitk_reduce_kernel<<<blocks, 256, 0, c->stream>>>(reinterpret_cast<const float4*>(c->splitk_ws), bias,
+    splitk_reduce_kernel<<<blocks, 256, 0, c->stream>>>(reinterpret_cast<const float4*>(ws), bias,
                                                        reinterpret_cast<float4*>(C), mn4, N / 4, splits, relu);
     c->launches++;
     DISN_CUDA_OK(cudaGetLastError());
@@ -354,8 +355,9 @@ static int launch_gemv(disn_ctx* c, const float* x, const float* W, const float*
   DISN_REQUIRE(B <= GEMV_MAXB && N % 4 == 0, "gemv: batch <= 8 and N % 4 == 0");
   int splits = (K + GEMV_KS - 1) / GEMV_KS;
   dim3 grid((N / 4 + 255) / 256, splits);
-  gemv_partial_kernel<<<grid, 256, 0, c->stream>>>(x, W, c->partial, B, K, N);
-  gemv_reduce_kernel<<<(B * N + 255) / 256, 256, 0, c->stream>>>(c->partial, bias, out, B, N, splits, relu);
+  float* partial = c->partial.get<float>();
+  gemv_partial_kernel<<<grid, 256, 0, c->stream>>>(x, W, partial, B, K, N);
+  gemv_reduce_kernel<<<(B * N + 255) / 256, 256, 0, c->stream>>>(partial, bias, out, B, N, splits, relu);
   c->launches += 2;
   DISN_CUDA_OK(cudaGetLastError());
   return 0;
@@ -413,40 +415,27 @@ static const char* kConvName[kNumConv] = {
     "vgg_16/conv5/conv5_3"};
 static const int kTapHW[5] = {224, 112, 56, 28, 14};
 
-void encoder_graph_reset(disn_ctx* c);
-
-void encoder_free(disn_ctx* c) {
-  encoder_graph_reset(c);      // the captured graph holds these buffers' addresses
-  auto fr = [](float*& p) { if (p) cudaFree(p); p = nullptr; };
-  fr(c->img_in); fr(c->img_rs); fr(c->act[0]); fr(c->act[1]);
-  for (int i = 0; i < 5; ++i) { fr(c->taps[i]); fr(c->proj[i]); }
-  fr(c->fc_a); fr(c->fc_b); fr(c->partial); fr(c->emb); fr(c->gbias); fr(c->pmap); fr(c->splitk_ws);
-  c->splitk_ws_elems = 0;
-  c->alloc_B = 0;
-}
-
 int encoder_alloc(disn_ctx* c, int B) {
   if (B <= c->alloc_B) return 0;
-  encoder_free(c);
-  const int V = c->cfg.vgg_in;
-  DISN_REQUIRE(V == 224, "vgg_in must be 224 (fc6 is a 7x7 VALID conv on the pool5 map)");
-  auto al = [&](float*& p, int64_t n) -> int { DISN_CUDA_OK(cudaMalloc(&p, n * sizeof(float))); return 0; };
-  int64_t Bn = B;
-  if (al(c->img_in, Bn * V * V * 4)) return -1;
-  if (al(c->img_rs, Bn * V * V * 3)) return -1;
-  for (int i = 0; i < 2; ++i) if (al(c->act[i], Bn * V * V * 64)) return -1;
+  const int64_t Bn = B, V = c->cfg.vgg_in;
+  std::vector<std::pair<DevBuf*, int64_t>> bufs = {{&c->img_in, Bn * V * V * 4}, {&c->img_rs, Bn * V * V * 3},
+                                                   {&c->act[0], Bn * V * V * 64}, {&c->act[1], Bn * V * V * 64}};
   for (int i = 0; i < 5; ++i) {
-    if (al(c->taps[i], Bn * kTapHW[i] * kTapHW[i] * kTapC[i])) return -1;
-    if (al(c->proj[i], Bn * kTapHW[i] * kTapHW[i] * kHidden)) return -1;
+    bufs.push_back({&c->taps[i], Bn * kTapHW[i] * kTapHW[i] * kTapC[i]});
+    bufs.push_back({&c->proj[i], Bn * kTapHW[i] * kTapHW[i] * kHidden});
   }
-  if (al(c->fc_a, Bn * 4096)) return -1;
-  if (al(c->fc_b, Bn * 4096)) return -1;
-  if (al(c->partial, (int64_t)((25088 + GEMV_KS - 1) / GEMV_KS) * Bn * 4096)) return -1;
-  if (al(c->emb, Bn * c->cfg.num_classes)) return -1;
-  if (al(c->gbias, Bn * kHidden)) return -1;
-  if (al(c->pmap, Bn * c->cfg.img_h * c->cfg.img_w * kHidden)) return -1;
-  c->splitk_ws_elems = Bn * 8 * 1024 * 1024;       // 32 MB per image of split-K partial sums
-  if (al(c->splitk_ws, c->splitk_ws_elems)) return -1;
+  bufs.insert(bufs.end(), {{&c->fc_a, Bn * 4096}, {&c->fc_b, Bn * 4096},
+                           {&c->partial, (int64_t)((25088 + GEMV_KS - 1) / GEMV_KS) * Bn * 4096},
+                           {&c->emb, Bn * c->cfg.num_classes}, {&c->gbias, Bn * kHidden},
+                           {&c->pmap, Bn * c->cfg.img_h * c->cfg.img_w * kHidden},
+                           {&c->splitk_ws, Bn * 8 * 1024 * 1024}});     // 32 MB per image of split-K partial sums
+  // all or nothing: every buffer is freed before any is allocated at the new size
+  encoder_graph_reset(c);      // the captured graph holds these buffers' addresses
+  for (auto& b : bufs) b.first->reset();
+  c->alloc_B = 0;
+  DISN_REQUIRE(V == 224, "vgg_in must be 224 (fc6 is a 7x7 VALID conv on the pool5 map)");
+  for (auto& b : bufs)
+    if (b.first->reserve(b.second * sizeof(float))) return -1;
   c->alloc_B = B;
   return 0;
 }
@@ -462,12 +451,16 @@ extern "C" int disn_debug_gemm(disn_ctx* c, const float* A, const float* Wt, con
   DISN_CUDA_OK(cudaSetDevice(c->cfg.device));
   if (encoder_alloc(c, 1)) return -1;
   const size_t a_elems = H ? (size_t)M * Cin : (size_t)M * K;
-  float *dA = nullptr, *dW = nullptr, *dB = nullptr, *dC = nullptr;
-  DISN_CUDA_OK(cudaMalloc(&dA, a_elems * 4)); DISN_CUDA_OK(cudaMalloc(&dW, (size_t)K * N * 4));
-  DISN_CUDA_OK(cudaMalloc(&dC, (size_t)M * N * 4));
+  DevBuf bA, bW, bB, bC;
+  if (bA.reserve(a_elems * 4) || bW.reserve((size_t)K * N * 4) || bC.reserve((size_t)M * N * 4)) return -1;
+  float *dA = bA.get<float>(), *dW = bW.get<float>(), *dC = bC.get<float>();
   DISN_CUDA_OK(cudaMemcpy(dA, A, a_elems * 4, cudaMemcpyHostToDevice));
   DISN_CUDA_OK(cudaMemcpy(dW, Wt, (size_t)K * N * 4, cudaMemcpyHostToDevice));
-  if (bias) { DISN_CUDA_OK(cudaMalloc(&dB, (size_t)N * 4)); DISN_CUDA_OK(cudaMemcpy(dB, bias, (size_t)N * 4, cudaMemcpyHostToDevice)); }
+  if (bias) {
+    if (bB.reserve((size_t)N * 4)) return -1;
+    DISN_CUDA_OK(cudaMemcpy(bB.get<float>(), bias, (size_t)N * 4, cudaMemcpyHostToDevice));
+  }
+  const float* dB = bB.get<float>();
   DISN_CUDA_OK(cudaDeviceSynchronize());   // pageable H2D copies above are not ordered against the ctx stream
   ConvGeom g{H, Wd, Cin};
   const int mode = H ? A_IM2COL : A_PLAIN;
@@ -484,9 +477,7 @@ extern "C" int disn_debug_gemm(disn_ctx* c, const float* A, const float* Wt, con
     }
   }
   c->cfg.precision = saved;
-  auto it = c->enc_tc_weights.find("debug_gemm");
-  if (it != c->enc_tc_weights.end()) { cudaFree(it->second); c->enc_tc_weights.erase(it); }
-  cudaFree(dA); cudaFree(dW); cudaFree(dB); cudaFree(dC);
+  c->enc_tc_weights.erase("debug_gemm");
   return rc;
 }
 #endif  // DISN_DIAGNOSTICS
@@ -494,7 +485,7 @@ namespace disn {
 
 static const float* wptr(disn_ctx* c, const std::string& name) {
   auto it = c->weights.find(name);
-  return it == c->weights.end() ? nullptr : it->second.ptr;
+  return it == c->weights.end() ? nullptr : it->second.data.get<float>();
 }
 
 int encoder_gemv(disn_ctx* c, const float* x, const float* W, const float* bias, float* out, int B, int K, int N, int relu) {
@@ -524,7 +515,7 @@ int encoder_run(disn_ctx* c, const float* imgs, int B, int H, int W, int C, bool
   DISN_REQUIRE(B >= 1 && B <= GEMV_MAXB, "batch must be in [1,8]");
   DISN_REQUIRE((int64_t)H * W <= (int64_t)c->cfg.vgg_in * c->cfg.vgg_in * 4 / 3, "input image too large");
   if (encoder_alloc(c, B)) return -1;
-  DISN_CUDA_OK(cudaMemcpyAsync(c->img_in, imgs, (size_t)B * H * W * C * sizeof(float),
+  DISN_CUDA_OK(cudaMemcpyAsync(c->img_in.get<float>(), imgs, (size_t)B * H * W * C * sizeof(float),
                                device_ptr ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, c->stream));
   const std::vector<int64_t> key = {B, H, W, C, (int64_t)embedding_only, (int64_t)c->cfg.precision};
   static const bool no_graph = getenv("DISN_NO_GRAPH") != nullptr;
@@ -578,22 +569,22 @@ static int encoder_body(disn_ctx* c, int B, int H, int W, int C, bool embedding_
                  std::string("missing weights for ") + nm);
   }
 
-  const float* x = c->img_in;
+  float *img_in = c->img_in.get<float>(), *img_rs = c->img_rs.get<float>();
+  const float* x = img_in;
   if (H != V || W != V) {  // model_normalization.py:65-72
-    resize_bilinear_tf_kernel<<<592, 256, 0, c->stream>>>(c->img_in, c->img_rs, B, H, W, C, V, V);
+    resize_bilinear_tf_kernel<<<592, 256, 0, c->stream>>>(img_in, img_rs, B, H, W, C, V, V);
     c->launches++;
-    x = c->img_rs;
+    x = img_rs;
   } else {
-    DISN_CUDA_OK(cudaMemcpyAsync(c->img_rs, c->img_in, (size_t)B * V * V * 3 * sizeof(float),
-                                 cudaMemcpyDeviceToDevice, c->stream));
-    x = c->img_rs;
+    DISN_CUDA_OK(cudaMemcpyAsync(img_rs, img_in, (size_t)B * V * V * 3 * sizeof(float), cudaMemcpyDeviceToDevice, c->stream));
+    x = img_rs;
   }
   // 13 convs + 5 pools (models/CNN/vgg.py:187-196)
   int pp = 0, tap = 0;
   for (int i = 0; i < kNumConv; ++i) {
     int hw = kConvHW[i];
     bool is_tap = (tap < 5 && kTapLayer[tap] == i);
-    float* y = is_tap ? c->taps[tap] : c->act[pp];
+    float* y = is_tap ? c->taps[tap].get<float>() : c->act[pp].get<float>();
     ConvGeom g{hw, hw, kConvCin[i]};
     if (gemm_any(c, std::string(kConvName[i]) + "/weights", A_IM2COL, x, wptr(c, std::string(kConvName[i]) + "/weights"),
                  wptr(c, std::string(kConvName[i]) + "/biases"), y, B * hw * hw, kConvCout[i], 9 * kConvCin[i], 1, g))
@@ -601,7 +592,7 @@ static int encoder_body(disn_ctx* c, int B, int H, int W, int C, bool embedding_
     x = y;
     if (!is_tap) pp ^= 1;
     if (is_tap) {
-      float* p = c->act[pp];
+      float* p = c->act[pp].get<float>();
       int64_t total = (int64_t)B * (hw / 2) * (hw / 2) * (kConvCout[i] / 4);
       int blocks = (int)std::min<int64_t>((total + 255) / 256, 148 * 8);
       maxpool2_kernel<<<blocks, 256, 0, c->stream>>>(reinterpret_cast<const float4*>(x), reinterpret_cast<float4*>(p),
@@ -613,11 +604,12 @@ static int encoder_body(disn_ctx* c, int B, int H, int W, int C, bool embedding_
     }
   }
   // fc6 (7x7 VALID == dense over the (y,x,c)-flattened 7x7x512 map), fc7, fc8 (linear)
-  if (launch_gemv(c, x, wptr(c, "vgg_16/fc6/weights"), wptr(c, "vgg_16/fc6/biases"), c->fc_a, B, 7 * 7 * 512, 4096, 1))
+  float *fc_a = c->fc_a.get<float>(), *fc_b = c->fc_b.get<float>(), *emb = c->emb.get<float>();
+  if (launch_gemv(c, x, wptr(c, "vgg_16/fc6/weights"), wptr(c, "vgg_16/fc6/biases"), fc_a, B, 7 * 7 * 512, 4096, 1))
     return -1;
-  if (launch_gemv(c, c->fc_a, wptr(c, "vgg_16/fc7/weights"), wptr(c, "vgg_16/fc7/biases"), c->fc_b, B, 4096, 4096, 1))
+  if (launch_gemv(c, fc_a, wptr(c, "vgg_16/fc7/weights"), wptr(c, "vgg_16/fc7/biases"), fc_b, B, 4096, 4096, 1))
     return -1;
-  if (launch_gemv(c, c->fc_b, wptr(c, "vgg_16/fc8/weights"), wptr(c, "vgg_16/fc8/biases"), c->emb, B, 4096,
+  if (launch_gemv(c, fc_b, wptr(c, "vgg_16/fc8/weights"), wptr(c, "vgg_16/fc8/biases"), emb, B, 4096,
                   c->cfg.num_classes, 0))
     return -1;
   if (embedding_only) {      // camera-pose net: only the VGG embedding is needed
@@ -625,8 +617,8 @@ static int encoder_body(disn_ctx* c, int B, int H, int W, int C, bool embedding_
     return 0;
   }
   // global-feature fold: gbias = emb * Wg[512:512+nc, :] + b   (models/sdfnet.py:78-85)
-  if (launch_gemv(c, c->emb, wptr(c, "sdfprediction/fold2/conv1/weights") + (int64_t)kHidden * kHidden,
-                  wptr(c, "sdfprediction/fold2/conv1/biases"), c->gbias, B, c->cfg.num_classes, kHidden, 0))
+  if (launch_gemv(c, emb, wptr(c, "sdfprediction/fold2/conv1/weights") + (int64_t)kHidden * kHidden,
+                  wptr(c, "sdfprediction/fold2/conv1/biases"), c->gbias.get<float>(), B, c->cfg.num_classes, kHidden, 0))
     return -1;
   // local-feature fold: proj_l = tap_l * Wl[512+off_l : 512+off_l+C_l, :]   (models/sdfnet.py:180-183)
   const float* wl = wptr(c, "sdfprediction_imgfeat/fold2/conv1/weights") + (int64_t)kHidden * kHidden;
@@ -634,32 +626,32 @@ static int encoder_body(disn_ctx* c, int B, int H, int W, int C, bool embedding_
   PmapLevels lv;
   for (int l = 0; l < 5; ++l) {
     int hw = kTapHW[l];
-    const float* src = c->taps[l];
+    const float* src = c->taps[l].get<float>();
     if (hw > c->cfg.img_h && c->cfg.img_h == c->cfg.img_w) {
       // resize and projection commute (both linear per channel): where the tap is LARGER than the 137x137 target (conv1_2,
       // 224x224) resize first -- the GEMM then has 2.7x fewer rows and the [B,224,224,512] intermediate (103 MB per image)
       // never exists.  This is also the reference's own order (model_normalization.py:171-172).
-      float* tmp = c->act[0];
+      float* tmp = c->act[0].get<float>();
       const int oh = c->cfg.img_h;
       const int64_t total = (int64_t)B * oh * oh * kTapC[l];
       resize_bilinear_tf_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, c->stream>>>(
-          c->taps[l], tmp, B, hw, hw, kTapC[l], oh, oh);
+          c->taps[l].get<float>(), tmp, B, hw, hw, kTapC[l], oh, oh);
       c->launches++;
       src = tmp;
       hw = oh;
     }
     ConvGeom g{0, 0, 0};
-    if (gemm_any(c, "proj" + std::to_string(l), A_PLAIN, src, wl + (int64_t)off * kHidden, nullptr, c->proj[l],
+    if (gemm_any(c, "proj" + std::to_string(l), A_PLAIN, src, wl + (int64_t)off * kHidden, nullptr, c->proj[l].get<float>(),
                  B * hw * hw, kHidden, kTapC[l], 0, g))
       return -1;
     off += kTapC[l];
-    lv.p[l] = c->proj[l];
+    lv.p[l] = c->proj[l].get<float>();
     lv.h[l] = hw;
   }
   {
     int64_t total = (int64_t)B * c->cfg.img_h * c->cfg.img_w * (kHidden / 4);
     int blocks = (int)std::min<int64_t>((total + 255) / 256, 148 * 16);
-    pmap_accumulate_kernel<<<blocks, 256, 0, c->stream>>>(lv, reinterpret_cast<float4*>(c->pmap), B, c->cfg.img_h,
+    pmap_accumulate_kernel<<<blocks, 256, 0, c->stream>>>(lv, reinterpret_cast<float4*>(c->pmap.get<float>()), B, c->cfg.img_h,
                                                           c->cfg.img_w);
     c->launches++;
   }

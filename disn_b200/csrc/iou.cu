@@ -152,48 +152,43 @@ extern "C" int disn_iou(disn_ctx* c, const float* verts1, int64_t nv1, const int
   const int64_t vox_words = (int64_t)VG * VG * VG / 32, n_occ = (int64_t)dim * dim * dim, occ_words = (n_occ + 31) / 32;
   const size_t bytes = (size_t)(nv1 + nv2) * 12 + (size_t)(nf1 + nf2) * 12 + (size_t)(vox_words + 2 * occ_words) * 4 + 16 +
                        (size_t)n_occ + 4096;
-  char* base = nullptr;
-  cudaError_t e = cudaMalloc(&base, bytes);
-  if (e != cudaSuccess) { set_error(std::string("cudaMalloc: ") + cudaGetErrorString(e)); return -1; }
-  auto fail = [&](const char* what, cudaError_t err) { set_error(std::string(what) + ": " + cudaGetErrorString(err)); cudaFree(base); return -1; };
-  char* p = base;
-  auto take = [&](size_t n) { char* r = p; p += (n + 255) / 256 * 256; return r; };
-  uint32_t* vox = reinterpret_cast<uint32_t*>(take(vox_words * 4));
-  uint32_t* occ[2] = {reinterpret_cast<uint32_t*>(take(occ_words * 4)), reinterpret_cast<uint32_t*>(take(occ_words * 4))};
-  unsigned long long* cnt = reinterpret_cast<unsigned long long*>(take(16));
-  uint8_t* unp = reinterpret_cast<uint8_t*>(take(n_occ));
+  DevBuf buf;
+  if (buf.reserve(bytes)) return -1;
+  uint32_t* vox = buf.take<uint32_t>(vox_words);
+  uint32_t* occ[2] = {buf.take<uint32_t>(occ_words), buf.take<uint32_t>(occ_words)};
+  unsigned long long* cnt = buf.take<unsigned long long>(2);
+  uint8_t* unp = buf.take<uint8_t>(n_occ);
   const double cell = 2.0 / (double)dim;                 // pymesh.VoxelGrid(2./dim)
   const int grid = c->num_sms * 8;
-  if ((e = cudaMemsetAsync(occ[0], 0, occ_words * 4, c->stream)) != cudaSuccess) return fail("memset", e);
-  if ((e = cudaMemsetAsync(occ[1], 0, occ_words * 4, c->stream)) != cudaSuccess) return fail("memset", e);
-  if ((e = cudaMemsetAsync(cnt, 0, 16, c->stream)) != cudaSuccess) return fail("memset", e);
+  DISN_CUDA_OK(cudaMemsetAsync(occ[0], 0, occ_words * 4, c->stream));
+  DISN_CUDA_OK(cudaMemsetAsync(occ[1], 0, occ_words * 4, c->stream));
+  DISN_CUDA_OK(cudaMemsetAsync(cnt, 0, 16, c->stream));
   for (int m = 0; m < 2; ++m) {
     const float* hv = m ? verts2 : verts1;
     const int32_t* hf = m ? faces2 : faces1;
     const int64_t nv = m ? nv2 : nv1, nf = m ? nf2 : nf1;
-    float* dv = reinterpret_cast<float*>(take((size_t)nv * 12));
-    int32_t* df = reinterpret_cast<int32_t*>(take((size_t)nf * 12));
-    if ((e = cudaMemcpyAsync(dv, hv, (size_t)nv * 12, cudaMemcpyHostToDevice, c->stream)) != cudaSuccess) return fail("copy", e);
-    if ((e = cudaMemcpyAsync(df, hf, (size_t)nf * 12, cudaMemcpyHostToDevice, c->stream)) != cudaSuccess) return fail("copy", e);
-    if ((e = cudaMemsetAsync(vox, 0, vox_words * 4, c->stream)) != cudaSuccess) return fail("memset", e);
+    float* dv = buf.take<float>((size_t)nv * 3);
+    int32_t* df = buf.take<int32_t>((size_t)nf * 3);
+    DISN_CUDA_OK(cudaMemcpyAsync(dv, hv, (size_t)nv * 12, cudaMemcpyHostToDevice, c->stream));
+    DISN_CUDA_OK(cudaMemcpyAsync(df, hf, (size_t)nf * 12, cudaMemcpyHostToDevice, c->stream));
+    DISN_CUDA_OK(cudaMemsetAsync(vox, 0, vox_words * 4, c->stream));
     voxelize_kernel<<<grid, 128, 0, c->stream>>>(dv, df, nf, cell, vox);
     corners_kernel<<<grid, 256, 0, c->stream>>>(vox, cell, dim, occ[m]);
     c->launches += 2;
   }
   iou_count_kernel<<<grid, 256, 0, c->stream>>>(occ[0], occ[1], occ_words, cnt);
   c->launches++;
-  if ((e = cudaGetLastError()) != cudaSuccess) return fail("launch", e);
+  DISN_CUDA_OK(cudaGetLastError());
   unsigned long long h[2] = {0, 0};
-  if ((e = cudaMemcpyAsync(h, cnt, 16, cudaMemcpyDeviceToHost, c->stream)) != cudaSuccess) return fail("copy", e);
+  DISN_CUDA_OK(cudaMemcpyAsync(h, cnt, 16, cudaMemcpyDeviceToHost, c->stream));
   for (int m = 0; m < 2; ++m) {
     uint8_t* out = m ? occ2_out : occ1_out;
     if (!out) continue;
     unpack_bits_kernel<<<grid, 256, 0, c->stream>>>(occ[m], n_occ, unp);
-    if ((e = cudaMemcpyAsync(out, unp, (size_t)n_occ, cudaMemcpyDeviceToHost, c->stream)) != cudaSuccess) return fail("copy", e);
-    if ((e = cudaStreamSynchronize(c->stream)) != cudaSuccess) return fail("sync", e);
+    DISN_CUDA_OK(cudaMemcpyAsync(out, unp, (size_t)n_occ, cudaMemcpyDeviceToHost, c->stream));
+    DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
   }
-  if ((e = cudaStreamSynchronize(c->stream)) != cudaSuccess) return fail("sync", e);
-  cudaFree(base);
+  DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
   *intersection = (int64_t)h[0];
   *uni = (int64_t)h[1];
   return 0;

@@ -602,20 +602,19 @@ int launch_var(disn_ctx* c, const PointJob& job, const SmallParams& sp, const vo
     DISN_CUDA_OK(cudaFuncSetAttribute(point_tc_kernel<kMode, kVar, kCorr>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     c->attr_done.insert(key);
   }
-  unsigned long long* dbg = nullptr;
+  DevBuf dbg;
   int expt = 0;
   if constexpr ((kVar & 1) != 0) {
     expt = getenv("DISN_TC_EXPT") ? atoi(getenv("DISN_TC_EXPT")) : 0;
-    DISN_CUDA_OK(cudaMalloc(&dbg, (size_t)pairs * 2 * (1 + 16 * W_NCLS) * sizeof(unsigned long long)));
-    DISN_CUDA_OK(cudaMemsetAsync(dbg, 0, (size_t)pairs * 2 * (1 + 16 * W_NCLS) * sizeof(unsigned long long), c->stream));
+    if (dbg.reserve((size_t)pairs * 2 * (1 + 16 * W_NCLS) * sizeof(unsigned long long))) return -1;
+    DISN_CUDA_OK(cudaMemsetAsync(dbg.get<void>(), 0, dbg.bytes(), c->stream));
   }
   point_tc_kernel<kMode, kVar, kCorr><<<pairs * 2, NTHREADS, smem, c->stream>>>(
-      job, sp, reinterpret_cast<const uint8_t*>(wpk), tiles_per_img, dbg, expt);
+      job, sp, reinterpret_cast<const uint8_t*>(wpk), tiles_per_img, dbg.get<unsigned long long>(), expt);
   if constexpr ((kVar & 1) != 0) {
     std::vector<unsigned long long> h((size_t)pairs * 2 * (1 + 16 * W_NCLS));
     DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
-    DISN_CUDA_OK(cudaMemcpy(h.data(), dbg, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    cudaFree(dbg);
+    DISN_CUDA_OK(cudaMemcpy(h.data(), dbg.get<void>(), h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     const int nc = pairs * 2;
     double sum = 0, mx = 0;
     for (int i = 0; i < nc; ++i) { sum += (double)h[i]; mx = std::max(mx, (double)h[i]); }
@@ -661,7 +660,8 @@ int tc_pack_weights(disn_ctx* c) {
       DISN_REQUIRE(it != c->weights.end(), "missing variable " + p + names[layer]);
       const int K = Ks[layer], N = Ns[layer];
       std::vector<float> w((size_t)K * N);   // rows 0..K-1 of the [Cin,Cout] matrix (point-feature part)
-      DISN_CUDA_OK(cudaMemcpyAsync(w.data(), it->second.ptr, w.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+      DISN_CUDA_OK(cudaMemcpyAsync(w.data(), it->second.data.get<float>(), w.size() * sizeof(float), cudaMemcpyDeviceToHost,
+                                   c->stream));
       DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
       for (int t = 0; t < K / 64; ++t)
         for (int nb = 0; nb < N / 256; ++nb, ++stage)
@@ -682,15 +682,8 @@ int tc_pack_weights(disn_ctx* c) {
     }
   }
   DISN_REQUIRE(stage == (size_t)2 * STAGES_PER_STREAM, "internal: stage count");
-  if (c->tc_weights_bytes != (int64_t)total) {
-    if (c->tc_weights) cudaFree(c->tc_weights);
-    if (c->tc_weights_f8) cudaFree(c->tc_weights_f8);
-    c->tc_weights = c->tc_weights_f8 = nullptr;
-    DISN_CUDA_OK(cudaMalloc(&c->tc_weights, total));
-    DISN_CUDA_OK(cudaMalloc(&c->tc_weights_f8, total));
-    c->tc_weights_bytes = (int64_t)total;
-  }
-  DISN_CUDA_OK(cudaMemcpyAsync(c->tc_weights, img.data(), total, cudaMemcpyHostToDevice, c->stream));
+  if (c->tc_weights.reserve(total) || c->tc_weights_f8.reserve(total)) return -1;
+  DISN_CUDA_OK(cudaMemcpyAsync(c->tc_weights.get<void>(), img.data(), total, cudaMemcpyHostToDevice, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));   // ordered on the ctx stream (see conv_tc_pack)
 
   // ---- DISN_PREC_F16F8 images: per (stage, CTA half): [fp16 W, SW128, 16 KB | e5m2(w.2^-s1), SW64, 8 KB |
@@ -706,7 +699,8 @@ int tc_pack_weights(disn_ctx* c) {
       auto it = c->weights.find(p + names[layer]);
       const int K = Ks[layer], N = Ns[layer];
       std::vector<float> w((size_t)K * N);
-      DISN_CUDA_OK(cudaMemcpyAsync(w.data(), it->second.ptr, w.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+      DISN_CUDA_OK(cudaMemcpyAsync(w.data(), it->second.data.get<float>(), w.size() * sizeof(float), cudaMemcpyDeviceToHost,
+                                   c->stream));
       DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
       double ss = 0;
       for (float v : w) ss += (double)v * v;
@@ -735,7 +729,7 @@ int tc_pack_weights(disn_ctx* c) {
           }
     }
   }
-  DISN_CUDA_OK(cudaMemcpyAsync(c->tc_weights_f8, img.data(), total, cudaMemcpyHostToDevice, c->stream));
+  DISN_CUDA_OK(cudaMemcpyAsync(c->tc_weights_f8.get<void>(), img.data(), total, cudaMemcpyHostToDevice, c->stream));
   DISN_CUDA_OK(cudaStreamSynchronize(c->stream));
 
   // host copy of the small per-stream parameters at the SB_* offsets (the kernel's __grid_constant__ parameter table)
@@ -748,7 +742,7 @@ int tc_pack_weights(disn_ctx* c) {
     for (const auto& e : small) {
       auto it = c->weights.find(p + e.name);
       DISN_REQUIRE(it != c->weights.end() && it->second.numel == e.n, "missing or mis-shaped variable " + p + e.name);
-      DISN_CUDA_OK(cudaMemcpyAsync(&c->tc_small[sidx][e.off], it->second.ptr, (size_t)e.n * sizeof(float),
+      DISN_CUDA_OK(cudaMemcpyAsync(&c->tc_small[sidx][e.off], it->second.data.get<float>(), (size_t)e.n * sizeof(float),
                                    cudaMemcpyDeviceToHost, c->stream));
     }
   }
@@ -758,7 +752,7 @@ int tc_pack_weights(disn_ctx* c) {
 
 int launch_point_tc(disn_ctx* c, const PointJob& job_in) {
   const bool f8 = c->cfg.precision == DISN_PREC_F16F8;
-  const void* wpk = f8 ? c->tc_weights_f8 : c->tc_weights;
+  const void* wpk = (f8 ? c->tc_weights_f8 : c->tc_weights).get<void>();
   DISN_REQUIRE(wpk != nullptr, "tensor-core weights not packed (call disn_finalize_weights)");
   static_assert(sizeof(SmallParams) == sizeof(c->tc_small), "small-parameter table layout");
   PointJob job = job_in;

@@ -124,11 +124,11 @@ extern "C" int disn_tc_stream_probe(int device) {
   using namespace disn;
   DISN_CUDA_OK(cudaSetDevice(device));
   const uint32_t image = 4u << 20;
-  uint8_t* src = nullptr;
-  unsigned long long* out = nullptr;
-  DISN_CUDA_OK(cudaMalloc(&src, image));
+  DevBuf bsrc, bout;
+  if (bsrc.reserve(image) || bout.reserve(512 * sizeof(unsigned long long))) return -1;
+  uint8_t* src = bsrc.get<uint8_t>();
+  unsigned long long* out = bout.get<unsigned long long>();
   DISN_CUDA_OK(cudaMemset(src, 1, image));
-  DISN_CUDA_OK(cudaMalloc(&out, 512 * sizeof(unsigned long long)));
   const int grid = 148;
   auto run = [&](int cs, int mode, uint32_t stage, int ns, int delay) -> int {
     const int smem = 2048 + (int)stage * ns + 1024;
@@ -181,7 +181,6 @@ extern "C" int disn_tc_stream_probe(int device) {
   }
   if (run(1, 0, 16384u, 6, 384)) return -1;     // consumer paced like the MMA at full rate (16 KB / 384 clk)
   if (run(1, 0, 32768u, 3, 768)) return -1;
-  cudaFree(src); cudaFree(out);
   fflush(stdout);
   return 0;
 }
@@ -260,15 +259,15 @@ __global__ void __launch_bounds__(32, 1) op_cost_kernel(unsigned long long* __re
 extern "C" int disn_tc_op_probe(int device) {
   using namespace disn;
   DISN_CUDA_OK(cudaSetDevice(device));
-  unsigned long long* d = nullptr;
-  DISN_CUDA_OK(cudaMalloc(&d, 64 * sizeof(unsigned long long)));
+  DevBuf bd;
+  if (bd.reserve(64 * sizeof(unsigned long long))) return -1;
+  unsigned long long* d = bd.get<unsigned long long>();
   DISN_CUDA_OK(cudaMemset(d, 0, 64 * sizeof(unsigned long long)));
   op_cost_kernel<<<1, 32>>>(d);
   DISN_CUDA_OK(cudaGetLastError());
   DISN_CUDA_OK(cudaDeviceSynchronize());
   unsigned long long h[64];
   DISN_CUDA_OK(cudaMemcpy(h, d, sizeof(h), cudaMemcpyDeviceToHost));
-  cudaFree(d);
   const char* names[14] = {"empty loop", "try_wait acquire (32 lanes)", "try_wait acquire (1 lane)", "try_wait relaxed (32 lanes)",
                            "try_wait relaxed (1 lane)", "test_wait (32 lanes)", "test_wait (1 lane)", "mbarrier.arrive (1 lane)",
                            "tcgen05.commit idle (1 lane)", "ld.volatile.shared (32 lanes)", "tcgen05.fence::after_thread_sync",

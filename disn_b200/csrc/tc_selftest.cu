@@ -109,10 +109,11 @@ extern "C" int disn_tc_selftest(int device, const float* A, const float* B, int 
       uint32_t off = tc::sw128_offset(row, k / 8) + (k % 8) * 2;
       memcpy(&bimg[(size_t)half * 128 * 128 + off], &v, 2);
     }
-  __nv_bfloat16* dA = nullptr; uint8_t* dB = nullptr; float* dD = nullptr;
-  DISN_CUDA_OK(cudaMalloc(&dA, a.size() * 2));
-  DISN_CUDA_OK(cudaMalloc(&dB, bimg.size()));
-  DISN_CUDA_OK(cudaMalloc(&dD, 2 * 128 * 128 * sizeof(float)));
+  DevBuf bA, bB, bD;
+  if (bA.reserve(a.size() * 2) || bB.reserve(bimg.size()) || bD.reserve(2 * 128 * 128 * sizeof(float))) return -1;
+  __nv_bfloat16* dA = bA.get<__nv_bfloat16>();
+  uint8_t* dB = bB.get<uint8_t>();
+  float* dD = bD.get<float>();
   DISN_CUDA_OK(cudaMemcpy(dA, a.data(), a.size() * 2, cudaMemcpyHostToDevice));
   DISN_CUDA_OK(cudaMemcpy(dB, bimg.data(), bimg.size(), cudaMemcpyHostToDevice));
   DISN_CUDA_OK(cudaMemset(dD, 0xff, 2 * 128 * 128 * sizeof(float)));
@@ -122,7 +123,6 @@ extern "C" int disn_tc_selftest(int device, const float* A, const float* B, int 
   DISN_CUDA_OK(cudaGetLastError());
   DISN_CUDA_OK(cudaDeviceSynchronize());
   DISN_CUDA_OK(cudaMemcpy(D_out, dD, 2 * 128 * 128 * sizeof(float), cudaMemcpyDeviceToHost));
-  cudaFree(dA); cudaFree(dB); cudaFree(dD);
   return 0;
 }
 
@@ -243,11 +243,13 @@ extern "C" int disn_tc_selftest_mixed(int device, const float* A16, const float*
       bimg[(size_t)half * 128 * 192 + 128 * 128 + tc::sw64_offset(row, k / 16) + (k % 16)] = q;
       B8q[n * 64 + k] = __half2float(__half(__nv_cvt_fp8_to_halfraw(q, __NV_E5M2)));
     }
-  __half* dA = nullptr; uint8_t *dA8 = nullptr, *dB = nullptr; float* dD = nullptr;
-  DISN_CUDA_OK(cudaMalloc(&dA, a16.size() * 2));
-  DISN_CUDA_OK(cudaMalloc(&dA8, a8.size()));
-  DISN_CUDA_OK(cudaMalloc(&dB, bimg.size()));
-  DISN_CUDA_OK(cudaMalloc(&dD, 2 * 128 * 128 * sizeof(float)));
+  DevBuf bA, bA8, bB, bD;
+  if (bA.reserve(a16.size() * 2) || bA8.reserve(a8.size()) || bB.reserve(bimg.size()) ||
+      bD.reserve(2 * 128 * 128 * sizeof(float)))
+    return -1;
+  __half* dA = bA.get<__half>();
+  uint8_t *dA8 = bA8.get<uint8_t>(), *dB = bB.get<uint8_t>();
+  float* dD = bD.get<float>();
   DISN_CUDA_OK(cudaMemcpy(dA, a16.data(), a16.size() * 2, cudaMemcpyHostToDevice));
   DISN_CUDA_OK(cudaMemcpy(dA8, a8.data(), a8.size(), cudaMemcpyHostToDevice));
   DISN_CUDA_OK(cudaMemcpy(dB, bimg.data(), bimg.size(), cudaMemcpyHostToDevice));
@@ -259,6 +261,5 @@ extern "C" int disn_tc_selftest_mixed(int device, const float* A16, const float*
   DISN_CUDA_OK(cudaGetLastError());
   DISN_CUDA_OK(cudaDeviceSynchronize());
   DISN_CUDA_OK(cudaMemcpy(D_out, dD, 2 * 128 * 128 * sizeof(float), cudaMemcpyDeviceToHost));
-  cudaFree(dA); cudaFree(dA8); cudaFree(dB); cudaFree(dD);
   return 0;
 }

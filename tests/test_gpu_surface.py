@@ -72,6 +72,47 @@ def test_intermediates_and_decoder_split_point(he_weights, precision):
         sess.close()
 
 
+def test_decoder_staging_survives_nn_distance(he_weights):
+    """nn_distance grows the context's device staging between decoder calls (eval_points_ex, point_img_feat,
+    eval_features): repeating those calls must give the same bits, and a larger one afterwards must match a fresh
+    context's."""
+    from disn_b200.engine import Engine
+    B = 2
+    imgs, tm = synth.synthetic_images(B, seed=31), synth.synthetic_trans_mats(B, seed=32)
+
+    def open_engine():
+        eng = Engine(device=0, precision="f16f8", max_batch=B)
+        eng.load_weights(he_weights)
+        eng.encode(imgs)
+        return eng
+
+    def decode(eng, N):
+        pts = np.random.default_rng(N).uniform(-1, 1, size=(B, N, 3)).astype(np.float32)
+        feat, uv = eng.point_img_feat(pts, tm)
+        return eng.eval_points_ex(pts, tm) + (feat, uv) + eng.eval_features(pts, eng.get_encoded(0), feat)
+
+    eng = open_engine()
+    try:
+        small = decode(eng, 64)
+        rng = np.random.default_rng(34)
+        a, b = (rng.uniform(-1, 1, size=(B, 20000, 3)).astype(np.float32) for _ in range(2))
+        d1, i1, d2, i2 = eng.nn_distance(a, b)     # 1.6 MB of staging: more than the decoder calls above needed
+        for k in (0, 777, 19999):
+            np.testing.assert_allclose(d1[1, k], ((b[1] - a[1, k]) ** 2).sum(-1).min(), rtol=1e-5, atol=1e-7)
+            np.testing.assert_allclose(d2[0, k], ((a[0] - b[0, k]) ** 2).sum(-1).min(), rtol=1e-5, atol=1e-7)
+        for got, want in zip(decode(eng, 64), small):
+            np.testing.assert_array_equal(got, want)
+        large = decode(eng, 1500)
+    finally:
+        eng.close()
+    fresh = open_engine()
+    try:
+        for got, want in zip(large, decode(fresh, 1500)):
+            np.testing.assert_array_equal(got, want)
+    finally:
+        fresh.close()
+
+
 def test_literal_reference_loop_equals_device_grid(he_weights, tmp_path):
     """create_sdf.py:241-285 replayed literally (tests/reference_loop.py) == one disn_eval_grid call, bit for bit."""
     from disn_b200 import create_sdf as cs
